@@ -7,6 +7,7 @@ one step = one closest-hit pass over 2048 x 2048 x 16 = 67,108,864 camera rays +
 With --gpus N the ONE ray set is split by ray index over the ranks (strong scaling), the BVH is built on rank 0 and broadcast once.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scene S] [--layout cwbvh|bvh] [--tree hq|sah] [--res R]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).
   value        rays of all ranks / max-over-ranks device time, ray records resident in HBM when the timed region starts
@@ -291,6 +292,32 @@ def parity_sample(args, verts, h_prim, h_shadow, hits, bits, m):
     return out
 
 
+# ---------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_RAYS, DUMP_SEED = 1 << 20, 20240917
+
+
+def dump_outputs(out_dir, hits, bits, blocks, n_total, rank, world):
+    """What the timed step handed back - the closest hit of every camera ray (t, u, v, prim) and the occlusion bit of every shadow
+    ray - for a fixed, seeded sample of DUMP_RAYS rays of the whole set (32 bytes a ray: 32 MB), one .npy per field, so that two
+    builds of the project can be compared output for output.  With --gpus N every rank writes its own rays (file suffix .rank<r>)."""
+    m = min(n_total, DUMP_RAYS)
+    pick = np.arange(n_total) if m == n_total else np.sort(np.random.default_rng(DUMP_SEED).choice(n_total, m, replace=False))
+    gidx, lidx, off = [np.zeros(0, np.int64)], [np.zeros(0, np.int64)], 0
+    for b0, bc in blocks:
+        lo, hi = np.searchsorted(pick, [b0, b0 + bc])
+        gidx.append(pick[lo:hi])
+        lidx.append(pick[lo:hi] - b0 + off)
+        off += bc
+    g, l = np.concatenate(gidx), np.concatenate(lidx)
+    arrays = {"ray_index": g.astype(np.float64), "hit_t": hits[l, 0], "hit_u": hits[l, 1], "hit_v": hits[l, 2],
+              "hit_prim": hits[l, 3].view(np.uint32).astype(np.float64),
+              "occluded": ((bits[l >> 5] >> (l & 31).astype(np.uint32)) & 1).astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = f".rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), np.ascontiguousarray(a))
+
+
 # ---------------------------------------------------------------------------------------------- our arm
 def run_ours(args):
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -455,6 +482,8 @@ def run_ours(args):
     torch.cuda.synchronize()
     bits_dev = d_bits.cpu().numpy().view(np.uint32)
     hits = d_hits.cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, hits, bits_dev, blocks, n_total, rank, world)
 
     # ---- extra (SURVEY 8(d) config 4): incoherent rays - one diffuse bounce off every camera hit (tiny_bvh_speedtest.cpp:564-587 with a
     # per-ray xorshift seeded by the global ray index), same index shard, device resident; reported beside the headline, not in it
@@ -623,7 +652,13 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the incoherent-ray section")
     ap.add_argument("--parity-rays", type=int, default=1 << 20)
     ap.add_argument("--cpu-sample-rays", type=int, default=1 << 23)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's hits and occlusion bits for a seeded "
+                    "sample of rays to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the engine's timed path returned: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

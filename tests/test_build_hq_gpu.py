@@ -94,15 +94,13 @@ def test_build_hq_is_deterministic(gpu):
 @pytest.mark.parametrize("scene", ["synthetic:5000", "bunny", "sponza"])
 def test_derived_layouts_build_hq(gpu, scene):
     """BVH_GPU::BuildHQ (:4588) and BVH8_CWBVH::BuildHQ (:5859): the SBVH pushed through the same converters."""
-    from oracle import refpy
-    if not refpy.available():
-        pytest.skip("needs oracle/_ref")
+    REF = util.reference()
     v, label = scenes.load_scene(scene)
-    ref = refpy.RefBVH(v, mode=2, threaded=False)
-    want = refpy.RefBVHGPU(ref).nodes
+    ref = REF.RefBVH(v, mode=2, threaded=False)
+    want = REF.RefBVHGPU(ref).nodes
     got = api.BVH_GPU().BuildHQ(v).download()
     assert got.shape == want.shape and np.array_equal(got.view(np.uint32), want.view(np.uint32)), f"{label}: BVH_GPU nodes differ"
-    cw = refpy.RefCWBVH(v, mode=1)
+    cw = REF.RefCWBVH(v, mode=1)
     e = api.BVH8_CWBVH().BuildHQ(v)
     nodes, tris = e.download()
     assert nodes.shape == cw.nodes.shape and np.array_equal(nodes.view(np.uint32), cw.nodes.view(np.uint32)), f"{label}: bvh8Data differs"
@@ -121,12 +119,10 @@ def test_derived_layouts_build_hq(gpu, scene):
 def test_indexed_geometry_builds(gpu, mode, method):
     """The ( vertices, indices, primCount ) overloads (tiny_bvh.h:889-900) through tbvh_build_indexed: same tree as the
     reference builds from the shared-vertex mesh, same hits."""
-    from oracle import refpy
     from tests.test_oracle_pin import indexed_mesh
-    if not refpy.available():
-        pytest.skip("needs oracle/_ref")
+    REF = util.reference()
     flat, verts, idx = indexed_mesh(20000, 43)
-    ref = refpy.RefBVH(verts, mode=mode, threaded=False, indices=idx)
+    ref = REF.RefBVH(verts, mode=mode, threaded=False, indices=idx)
     e = getattr(api.BVH(), method)(verts, indices=idx)
     nodes, pidx = e.download()
     assert e.info().prim_count == 20000

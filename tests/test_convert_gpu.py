@@ -9,6 +9,7 @@ from tests import golden_util as G
 from tests import util
 
 pytestmark = pytest.mark.gpu
+REF = util.reference()
 
 
 def diff_nodes(got, want, words):
@@ -27,14 +28,13 @@ def test_bvh_gpu_conversion_matches_golden(gpu, path):
     diff_nodes(e.download(), g["nodes_gpu"].view(np.uint8).view(api.NODE64).reshape(-1), 16)
 
 
-@pytest.mark.skipif(not refpy.available(), reason="needs oracle/_ref")
 @pytest.mark.parametrize("ntris,seed", [(5, 51), (999, 52), (120000, 53)])
 @pytest.mark.parametrize("flavour", [BUILD_REFERENCE, BUILD_AVX])
 def test_bvh_gpu_conversion_matches_reference(gpu, ntris, seed, flavour):
     """flavour AVX = BVH_GPU::Build itself (BuildDefault -> BuildAVX, then ConvertFrom); REFERENCE = ConvertFrom(BVH::Build)."""
     v = scenes.procedural_scene(ntris, seed)
-    ref = refpy.RefBVH(v, mode=1 if flavour == BUILD_AVX else 0, threaded=False)
-    want = refpy.RefBVHGPU(ref).nodes
+    ref = REF.RefBVH(v, mode=1 if flavour == BUILD_AVX else 0, threaded=False)
+    want = REF.RefBVHGPU(ref).nodes
     e = api.BVH_GPU()
     e.build_flavour = flavour
     e.Build(v)
@@ -71,14 +71,32 @@ def diff_blob(got, want, name, row_bytes):
     assert bad.size == 0, f"{name}: {bad.size} of {a.shape[0]} records differ, first {bad[:6]}\\n got  {a[bad[0]].view(np.uint32)}\\n want {b[bad[0]].view(np.uint32)}"
 
 
-@pytest.mark.skipif(not refpy.available(), reason="needs oracle/_ref")
+@pytest.mark.parametrize("path", [p for p in G.golden_files() if "cwbvh_nodes" in np.load(p).files], ids=lambda p: p.split("/")[-1])
+def test_cwbvh_conversion_matches_golden(gpu, path):
+    """The reference's BVH8_CWBVH chain over the scalar BVH::Build tree and its CPU walk, as recorded in the golden vectors
+    (tools/make_golden.py): the device build + conversion byte for byte, the device walk bit for bit."""
+    from tinybvh_b200 import rays as R
+    g = G.load(path)
+    e = api.BVH8_CWBVH()
+    e.build_flavour = BUILD_REFERENCE
+    e.Build(g["verts"])
+    nodes, tris = e.download()
+    diff_blob(nodes, g["cwbvh_nodes"], "bvh8Data (80-byte nodes)", 80)
+    diff_blob(tris, g["cwbvh_tris"], "bvh8Tris (48-byte triangles)", 48)
+    lo, hi = scenes.scene_bounds(g["verts"])
+    res = int(round((g["cwbvh_primary_hit"].shape[0] // 4) ** 0.5))
+    r = R.primary_rays(*R.bounds_camera(lo, hi, "outside"), res, res, 4)
+    e.Intersect(r)
+    assert np.array_equal(G.hits_as_u32(r), g["cwbvh_primary_hit"])
+
+
 @pytest.mark.parametrize("ntris,seed", [(1, 61), (3, 62), (4, 63), (40, 64), (2000, 65), (60000, 66)])
 @pytest.mark.parametrize("flavour", [BUILD_REFERENCE, BUILD_AVX])
 def test_cwbvh_conversion_matches_reference(gpu, ntris, seed, flavour):
     """flavour AVX: byte-identical to BVH8_CWBVH::Build itself (mode 0: BuildDefault = BuildAVX, Compact, SplitLeafs, collapse,
     encode); REFERENCE: the same chain over the scalar BVH::Build tree (mode 2)."""
     v = scenes.procedural_scene(ntris, seed)
-    cw = refpy.RefCWBVH(v, mode=0 if flavour == BUILD_AVX else 2)
+    cw = REF.RefCWBVH(v, mode=0 if flavour == BUILD_AVX else 2)
     e = api.BVH8_CWBVH()
     e.build_flavour = flavour
     e.Build(v)
@@ -87,11 +105,10 @@ def test_cwbvh_conversion_matches_reference(gpu, ntris, seed, flavour):
     diff_blob(tris, cw.tris, "bvh8Tris (48-byte triangles)", 48)
 
 
-@pytest.mark.skipif(not refpy.available(), reason="needs oracle/_ref")
 @pytest.mark.parametrize("scene", ["bunny", "sponza"])
 def test_cwbvh_conversion_fixtures(gpu, scene):
     v, label = scenes.load_scene(scene)
-    cw = refpy.RefCWBVH(v, mode=0)      # BVH8_CWBVH::Build as the reference runs it (threaded BuildAVX underneath)
+    cw = REF.RefCWBVH(v, mode=0)      # BVH8_CWBVH::Build as the reference runs it (threaded BuildAVX underneath)
     e = api.BVH8_CWBVH().Build(v)
     nodes, tris = e.download()
     diff_blob(nodes, cw.nodes, label + " bvh8Data", 80)

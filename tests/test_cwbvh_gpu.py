@@ -7,11 +7,11 @@ BVH::Build tree).  Two checks per ray set:
 import numpy as np
 import pytest
 
-from oracle import refpy
 from tinybvh_b200 import api, rays as R, scenes
 from tests import util
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not refpy.available(), reason="needs oracle/_ref (reference CWBVH builder)")]
+pytestmark = pytest.mark.gpu
+REF = util.reference()
 
 
 def check(e, cw, o, rays_in, verts, label):
@@ -60,7 +60,7 @@ def check_occlusion(e, cw, o, shadow, label):
 @pytest.mark.parametrize("ntris,seed,res", [(30000, 31, 96), (900, 32, 64), (20, 33, 32)])
 def test_cwbvh_seeded(gpu, ntris, seed, res):
     v = scenes.procedural_scene(ntris, seed)
-    cw = refpy.RefCWBVH(v, mode=2)
+    cw = REF.RefCWBVH(v, mode=2)
     o = util.oracle_bvh(v)
     e = api.BVH8_CWBVH().upload(cw.nodes, cw.tris)
     sets, bounds = util.ray_sets(v, res=res)
@@ -75,7 +75,7 @@ def test_cwbvh_seeded(gpu, ntris, seed, res):
 @pytest.mark.parametrize("scene", ["bunny", "sponza"])
 def test_cwbvh_fixtures(gpu, scene):
     v, label = scenes.load_scene(scene)
-    cw = refpy.RefCWBVH(v, mode=2)
+    cw = REF.RefCWBVH(v, mode=2)
     o = util.oracle_bvh(v)
     e = api.BVH8_CWBVH().upload(cw.nodes, cw.tris)
     lo, hi = scenes.scene_bounds(v)

@@ -389,16 +389,16 @@ def test_port_cwbvh_matches_reference(ntris, cw_mode, bvh_mode):
     assert np.array_equal(G.hits_as_u32(a), G.hits_as_u32(c))
 
 
-@pytest.mark.skipif(not refpy.available(), reason="oracle/_ref not built (needs /root/reference)")
 @pytest.mark.parametrize("ntris,seed,res,primary,diffuse", [(30000, 31, 96, 0, 8), (900, 32, 64, 69, 0), (20, 33, 32, 0, 0)])
 def test_reference_layouts_disagree_on_a_pinned_set_of_rays(ntris, seed, res, primary, diffuse):
     """The tie audit of SURVEY 8(c), pinned: on the seeded scenes of tests/test_cwbvh_gpu.py the reference's own CWBVH walk
     (BVH8_CWBVH::Intersect) and its BVH walk (BVH::Intersect) of the same triangles disagree on exactly this many rays (exact-distance ties;
     rays with a zero direction component, whose quantised plane distances overflow in the wide walk).  The GPU test then requires the engine's
-    CWBVH kernel to differ from BVH::Intersect on exactly the same rays as the reference's walk does - so these counts are the engine's too."""
+    CWBVH kernel to differ from BVH::Intersect on exactly the same rays as the reference's walk does - so these counts are the engine's too.
+    The counts were recorded from the compiled reference; without oracle/_ref the port's restatement of both walks must reproduce them."""
     from tests import util
     v = scenes.procedural_scene(ntris, seed)
-    cw, o = refpy.RefCWBVH(v, mode=2), util.oracle_bvh(v)
+    cw, o = util.reference().RefCWBVH(v, mode=2), util.oracle_bvh(v)
     sets, bounds = util.ray_sets(v, res=res)
     dis = lambda a, b: int(((a["prim"] != b["prim"]) | (a["t"].view(np.uint32) != b["t"].view(np.uint32))).sum())
     a, b = sets["primary"].copy(), sets["primary"].copy()

@@ -16,13 +16,11 @@ def words(r):
 
 @pytest.mark.parametrize("n_inst,builder", [(40, "Build"), (1, "Build"), (300, "BuildAVX"), (40, "BuildHQ")])
 def test_tlas_matches_reference(gpu, n_inst, builder):
-    from oracle import refpy
-    if not refpy.available():
-        pytest.skip("needs oracle/_ref")
+    REF = util.reference()
     v, inst, O, D = tlas_case(91, n_inst)
     mode = {"Build": 0, "BuildAVX": 1, "BuildHQ": 2}[builder]
     inst_ref = inst.copy()
-    ref = refpy.RefTLAS(inst_ref, [refpy.RefBVH(x, mode=mode, threaded=False) for x in v])   # Update()s inst_ref in place
+    ref = REF.RefTLAS(inst_ref, [REF.RefBVH(x, mode=mode, threaded=False) for x in v])   # Update()s inst_ref in place
     blas = [getattr(api.BVH(), builder)(x) for x in v]
     t = api.TLAS().Build(inst, blas)                                                         # the engine Update()s inst in place
     assert inst.tobytes() == inst_ref.tobytes(), "BLASInstance::Update differs"
@@ -42,13 +40,33 @@ def test_tlas_matches_reference(gpu, n_inst, builder):
     assert hit.sum() > 1000
 
 
+def test_tlas_matches_golden_vectors(gpu):
+    """The reference's TLAS path as recorded in tests/golden/tlas (tools/make_golden.py make_tlas): BLASInstance::Update, the TLAS tree,
+    IntersectTLAS hits (inst, t, u, v, prim) and IsOccludedTLAS bits for two ray masks."""
+    import os
+    from oracle import refpy
+    from tests import golden_util as G
+    g = dict(np.load(os.path.join(G.GOLDEN, "tlas", "tlas_24.npz")))
+    inst = g["instances_raw"].view(refpy.BLAS_INSTANCE).reshape(-1).copy()
+    t = api.TLAS().Build(inst, [api.BVH().Build(g["verts0"]), api.BVH().Build(g["verts1"])])
+    assert np.array_equal(inst.view(np.uint32).reshape(-1, 48), g["instances"]), "BLASInstance::Update differs"
+    nodes, idx = t.download()
+    assert np.array_equal(nodes.view(np.uint32).reshape(-1, 8), g["tlas_nodes"]) and np.array_equal(idx, g["tlas_prim_idx"]), "TLAS tree differs"
+    for mask in (1, 2):
+        r = np.zeros(g["rays_O"].shape[0], R.RAY_DTYPE)
+        r["O"], r["D"], r["rD"], r["t"], r["mask"] = g["rays_O"], g["rays_D"], g["rays_rD"], g["rays_tmax"], mask
+        sh = r.copy()
+        sh["t"] = 150.0
+        t.Intersect(r)
+        assert np.array_equal(words(r), g[f"hit_mask{mask}"]), f"closest hits differ (ray mask {mask:#x})"
+        assert np.array_equal(t.IsOccluded(sh), g[f"occluded_mask{mask}"])
+
+
 def test_tlas_device_rays_and_errors(gpu):
     import torch
-    from oracle import refpy
-    if not refpy.available():
-        pytest.skip("needs oracle/_ref")
+    REF = util.reference()
     v, inst, O, D = tlas_case(93, 24)
-    ref = refpy.RefTLAS(inst, [refpy.RefBVH(x, mode=0, threaded=False) for x in v])
+    ref = REF.RefTLAS(inst, [REF.RefBVH(x, mode=0, threaded=False) for x in v])
     blas = [api.BVH().Build(x) for x in v]
     t = api.TLAS().Build(inst, blas, update=False)   # records already updated by the reference: the "blasses == 0" contract
     rays = R.make_rays(O, D)
@@ -68,11 +86,9 @@ def test_tlas_device_rays_and_errors(gpu):
 
 def test_tlas_instance_bits_in_prim(gpu):
     """A host program compiled with INST_IDX_BITS 10 (the speedtest's setting): the instance rides in the top bits of hit.prim."""
-    from oracle import refpy
-    if not refpy.available():
-        pytest.skip("needs oracle/_ref")
+    REF = util.reference()
     v, inst, O, D = tlas_case(95, 30)
-    ref = refpy.RefTLAS(inst, [refpy.RefBVH(x, mode=0, threaded=False) for x in v])
+    ref = REF.RefTLAS(inst, [REF.RefBVH(x, mode=0, threaded=False) for x in v])
     t = api.TLAS().Build(inst, [api.BVH().Build(x) for x in v])
     rays = R.make_rays(O, D)
     want, got = rays.copy(), rays.copy()

@@ -13,6 +13,81 @@ def oracle_bvh(verts):
     return portpy.PortBVH(verts)
 
 
+class PortReference:
+    """The reference objects of oracle/refpy.py that the GPU parity tests use, restated on the plain-C port (oracle/tbvh_oracle*.c).
+    The port is pinned bit for bit to the reference by tests/test_oracle_pin.py (committed golden vectors everywhere, the compiled
+    reference where oracle/_ref exists), so a checkout without the compiled reference still runs every parity check that the port
+    can restate.  Not restated: the threaded builders' node numbering and BVH::Intersect's cost return value."""
+
+    class RefBVH:
+        """mode 0 BVH::Build, 1 BuildAVX, 2 BuildHQ + Compact.  The ( vertices, indices ) overloads build the tree of the flat soup
+        verts[indices] (test_reference_indexed_build_equals_flat_build)."""
+
+        def __init__(self, verts, mode=0, threaded=False, indices=None):
+            assert not threaded, "the port numbers nodes as the single-threaded builders do"
+            v = np.ascontiguousarray(verts, np.float32).reshape(-1, 4)
+            self.verts = v if indices is None else np.ascontiguousarray(v[np.asarray(indices, np.int64).reshape(-1)])
+            if mode == 2:
+                nodes, idx, self.idx_count = portpy.build_hq(self.verts)
+                self.port = portpy.PortBVH(self.verts, nodes=nodes, prim_idx=idx)
+            else:
+                self.port = portpy.PortBVH(self.verts, avx=mode == 1)
+                self.idx_count = self.port.prim_idx.shape[0]
+            self.nodes, self.prim_idx, self.used_nodes = self.port.nodes, self.port.prim_idx, self.port.used_nodes
+
+        def intersect(self, rays, threads=0):
+            return self.port.intersect(rays, threads)
+
+        def occluded(self, rays, threads=0):
+            return self.port.occluded(rays, threads)
+
+    class RefBVHGPU:
+        def __init__(self, bvh):
+            self.nodes = bvh.port.to_bvh_gpu()
+
+    class RefCWBVH:
+        """mode 0 BVH8_CWBVH::Build (the chain over the BuildAVX tree), 1 BuildHQ (over the SBVH), 2 the chain over BVH::Build's tree."""
+
+        def __init__(self, verts, mode=2):
+            self.src = PortReference.RefBVH(verts, mode={0: 1, 1: 2, 2: 0}[mode])
+            used = int(self.src.nodes["triCount"].sum())
+            self.port = portpy.PortCWBVH(self.src.nodes, self.src.prim_idx[:used], self.src.verts, idx_count=self.src.idx_count)
+            self.nodes, self.tris = self.port.nodes, self.port.tris
+
+        def source_bvh(self):
+            return self.src
+
+        def intersect(self, rays, threads=0):
+            return self.port.intersect(rays)
+
+    class RefTLAS:
+        """BVH::Build( BLASInstance*, .. ): BLASInstance::Update of every record in place, then the BVH::Build tree over the instance boxes
+        (a 'triangle' (min, max, min) has exactly that box), walked by IntersectTLAS / IsOccludedTLAS."""
+
+        def __init__(self, instances, blasses):
+            lo = np.stack([b.nodes[0]["aabbMin"] for b in blasses])[instances["blasIdx"]]
+            hi = np.stack([b.nodes[0]["aabbMax"] for b in blasses])[instances["blasIdx"]]
+            portpy.instance_update(instances, lo, hi)
+            boxes = np.zeros((instances.shape[0] * 3, 4), np.float32)
+            boxes[0::3, :3], boxes[1::3, :3], boxes[2::3, :3] = instances["aabbMin"], instances["aabbMax"], instances["aabbMin"]
+            self.tlas = portpy.PortBVH(boxes)
+            self.port = portpy.PortTLAS(self.tlas.nodes, self.tlas.prim_idx, instances, [b.port for b in blasses])
+
+        def bvh(self):
+            return self.tlas
+
+        def intersect(self, rays, threads=0):
+            return self.port.intersect(rays)
+
+        def occluded(self, rays, threads=0):
+            return self.port.occluded(rays)
+
+
+def reference():
+    """The compiled reference (oracle/refpy) when oracle/_ref exists, else its restatement on the pinned port."""
+    return refpy if refpy.available() else PortReference
+
+
 def small_scene(ntris=6000, seed=7):
     return scenes.procedural_scene(ntris, seed)
 
