@@ -74,15 +74,12 @@ int tbvh_device_count( void );
  * are read by the device's DMA engine from local memory instead of across the socket interconnect. */
 int tbvh_device_numa_node( int device );
 int tbvh_bind_thread_to_device( int device );
-/* tuning knobs (no reference counterpart; defaults are the measured best): "trace_variant" 0 = generic BVH2 kernel,
- * 3 = octant-switch, 4 = persistent warps; "small_t" builder switch point (8..256); "d2h_mode" / "h2d_split" / "host_path"
- * select how the host-buffer path moves ray records and hits across PCIe ("host_path" 0 = copy engine 2D copies, the default;
- * 1 = gather kernel over the pinned mapping; "d2h_mode" 0 = 2D copy of the 16-byte hits into the records, 1 = bytes 0..63 of every record return (full cache lines), 2 = packed copy + host
- * threads scatter, 3 = scatter kernel over
- * the pinned mapping; "h2d_split" 1..4 inbound streams per chunk; "chunk_rays" rays per pipeline chunk, default 524288).
- * Environment variables TBVH_<KEY> set the defaults at context creation.  BuildHQ: "hq_small" (fragments below which a subtree goes to the warp kernel, default 16),
- * "hq_cluster" (largest thread-block cluster per node, 1..16).  "inst_idx_bits": the host program's INST_IDX_BITS (see
- * tbvh_build_tlas). */
+/* context options (no reference counterpart).  Three keys; any other is TBVH_E_ARG:
+ *  "inst_idx_bits"  the host program's INST_IDX_BITS, where a TLAS hit stores its instance (default 32, see tbvh_build_tlas)
+ *  "small_t"        BVH::Build: subtrees of at most this many primitives are built by one warp each (8..128, default 128);
+ *                   every value gives the same tree
+ *  "build_mode"     BVH::Build large phase: 0 = one persistent cooperative launch (the default), 1 = one launch per stage and
+ *                   level (what a device that refuses the cooperative launch runs); both give the same tree */
 int tbvh_set_option( tbvh_ctx ctx, const char* key, int value );
 /* pinned host memory for ray buffers (replaces tinybvh::malloc64 / BVHContext::malloc for rays, tiny_bvh.h:261-292, 763-768).
  * The pages are taken from the NUMA node of the current CUDA device (tbvh_host_alloc) or of `device` (_near); buffers of 8 MiB and more
@@ -182,8 +179,8 @@ int tbvh_download_cwbvh( tbvh_bvh bvh, void* bvh8_data, void* bvh8_tris, int spa
  * host records, in place - copies bytes 0..63 in, writes t,u,v,prim back to bytes 48..63 of every record. */
 int tbvh_intersect( tbvh_bvh bvh, int layout, void* rays, uint32_t stride, uint64_t n );
 /* same traversal, hits delivered as a packed array of 16-byte (t,u,v,prim) records instead of being scattered into the
- * 128-byte ray records: the return trip becomes one contiguous copy per chunk (the in-place form pays a strided
- * 16-byte-row copy; see DESIGN.md 4.5).  `rays` is not modified. */
+ * 128-byte ray records: the return trip becomes one contiguous copy per chunk (the in-place form returns bytes 0..63
+ * of every record in a strided copy; see DESIGN.md 4.5).  `rays` is not modified. */
 int tbvh_intersect_packed( tbvh_bvh bvh, int layout, const void* rays, uint32_t stride, uint64_t n, void* hits );
 /* BVH::IsOccluded( const Ray& ) tiny_bvh.h:3382 / isoccluded_cwbvh (traverse_cwbvh.cl:343) for a batch:
  * bits[i>>5] bit (i&31) = occluded; (n+31)/32 words are written. */

@@ -1,5 +1,6 @@
-"""Every tuning variant (tbvh_set_option) must give the oracle's results: the traversal-kernel variants change which
-lane / code path runs a ray, never its arithmetic or order; the host-path modes change how bytes cross PCIe."""
+"""The shipped traversal and host-buffer paths give the oracle's results on every route a batch can take (host and device
+buffers, pinned and pageable memory, packed and in-place hits, several pipeline chunks), and the context options that
+remain (tbvh_set_option: small_t, build_mode) change how the tree is built, never the tree."""
 import numpy as np
 import pytest
 
@@ -23,52 +24,48 @@ def world():
     return v, sets["primary"], d, want
 
 
-@pytest.mark.parametrize("variant", [0, 3, 4])
-def test_trace_variants_are_bit_exact(gpu, world, variant):
+def test_bvh2_traversal_is_bit_exact(gpu, world):
     v, primary, d, want = world
     import torch
-    api.set_option("trace_variant", variant)
-    try:
-        e = api.BVH().Build(v)
-        for name, rays in (("primary", primary), ("diffuse", d["diffuse"])):
-            got = rays.copy()
-            e.Intersect(got)
-            assert util.compare_hits(got, want[name]) == ZERO, f"variant {variant} {name}"
-            # device path with a ragged count (persistent kernel tail handling)
-            m = rays.shape[0] - 37
-            dev = torch.from_numpy(R.gpu_records(rays[:m]).view(np.uint8).reshape(-1, 64).copy()).cuda()
-            hits = torch.zeros((m, 4), dtype=torch.float32, device="cuda")
-            e.Intersect(dev, hits=hits)
-            torch.cuda.synchronize()
-            h = hits.cpu().numpy()
-            assert np.array_equal(h[:, 0].view(np.uint32), want[name]["t"][:m].view(np.uint32))
-            assert np.array_equal(h[:, 3].view(np.uint32), want[name]["prim"][:m])
-        assert np.array_equal(e.IsOccluded(d["shadow"]), want["shadow_bits"]), f"variant {variant} occlusion"
-        m = d["shadow"].shape[0] - 37
-        assert np.array_equal(e.IsOccluded(d["shadow"][:m].copy()), util.oracle_bvh(v).occluded(d["shadow"][:m].copy()))
-    finally:
-        api.set_option("trace_variant", 3)
+    e = api.BVH().Build(v)
+    for name, rays in (("primary", primary), ("diffuse", d["diffuse"])):
+        got = rays.copy()
+        e.Intersect(got)
+        assert util.compare_hits(got, want[name]) == ZERO, name
+        # device path with a ragged count (a partial last warp and block)
+        m = rays.shape[0] - 37
+        dev = torch.from_numpy(R.gpu_records(rays[:m]).view(np.uint8).reshape(-1, 64).copy()).cuda()
+        hits = torch.zeros((m, 4), dtype=torch.float32, device="cuda")
+        e.Intersect(dev, hits=hits)
+        torch.cuda.synchronize()
+        h = hits.cpu().numpy()
+        assert np.array_equal(h[:, 0].view(np.uint32), want[name]["t"][:m].view(np.uint32))
+        assert np.array_equal(h[:, 3].view(np.uint32), want[name]["prim"][:m])
+    assert np.array_equal(e.IsOccluded(d["shadow"]), want["shadow_bits"]), "occlusion"
+    m = d["shadow"].shape[0] - 37
+    assert np.array_equal(e.IsOccluded(d["shadow"][:m].copy()), util.oracle_bvh(v).occluded(d["shadow"][:m].copy()))
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2, 3])
-def test_host_path_modes_return_the_same_hits(gpu, world, mode):
+def test_host_path_returns_the_same_hits_from_every_buffer(gpu, world):
     v, primary, d, want = world
-    api.set_option("d2h_mode", mode)
-    try:
-        e = api.BVH().Build(v)
-        n = primary.shape[0]
-        pinned = api.pinned_empty(n, R.RAY_DTYPE)
-        pinned[:] = primary
-        e.Intersect(pinned)
-        assert util.compare_hits(pinned, want["primary"]) == ZERO, f"d2h_mode {mode} (pinned)"
-        pageable = primary.copy()
-        e.Intersect(pageable)
-        assert util.compare_hits(pageable, want["primary"]) == ZERO, f"d2h_mode {mode} (pageable)"
-        hits = e.IntersectPacked(primary)   # packed return path: rays untouched, 16-byte hits
-        assert np.array_equal(hits["t"].view(np.uint32), want["primary"]["t"].view(np.uint32)) and np.array_equal(hits["prim"], want["primary"]["prim"])
-        api.pinned_free(pinned)
-    finally:
-        api.set_option("d2h_mode", 1)
+    e = api.BVH().Build(v)
+    n = primary.shape[0]
+    pinned = api.pinned_empty(n, R.RAY_DTYPE)
+    pinned[:] = primary
+    e.Intersect(pinned)
+    assert util.compare_hits(pinned, want["primary"]) == ZERO, "pinned"
+    pageable = primary.copy()
+    e.Intersect(pageable)
+    assert util.compare_hits(pageable, want["primary"]) == ZERO, "pageable"
+    hits = e.IntersectPacked(primary)   # packed return path: rays untouched, 16-byte hits
+    assert np.array_equal(hits["t"].view(np.uint32), want["primary"]["t"].view(np.uint32)) and np.array_equal(hits["prim"], want["primary"]["prim"])
+    api.pinned_free(pinned)
+
+
+def test_retired_option_keys_are_rejected(gpu):
+    for key in ("trace_variant", "d2h_mode", "chunk_rays"):
+        with pytest.raises(api.TbvhError):
+            api.set_option(key, 0)
 
 
 @pytest.mark.parametrize("small_t", [8, 64, 256])
@@ -83,9 +80,9 @@ def test_builder_switch_point_does_not_change_the_tree(gpu, small_t):
         api.set_option("small_t", 128)
 
 
-def test_long_host_batches_under_every_variant(gpu):
-    """Host batches longer than a pipeline chunk, several chunks in flight on different streams: the persistent-warp variant pulls
-    rays off a counter that must belong to ONE launch, and statistics must add up over the chunks of one call."""
+def test_long_host_batches(gpu):
+    """Host batches longer than a pipeline chunk, several chunks in flight on different streams: every chunk's hits and
+    occlusion words land in the right records, and statistics add up over the chunks of one call."""
     v = scenes.procedural_scene(30000, 73)
     o = util.oracle_bvh(v)
     lo, hi = scenes.scene_bounds(v)
@@ -95,15 +92,10 @@ def test_long_host_batches_under_every_variant(gpu):
     sh = util.derived_sets(want, v, (lo, hi))["shadow"]
     want_bits = o.occluded(sh, threads=0)
     e = api.BVH().Build(v)
-    for variant in (3, 4, 0):
-        api.set_option("trace_variant", variant)
-        try:
-            got = rays.copy()
-            e.Intersect(got)
-            assert util.compare_hits(got, want) == ZERO, f"variant {variant}"
-            assert np.array_equal(e.IsOccluded(sh), want_bits), f"variant {variant} occlusion"
-        finally:
-            api.set_option("trace_variant", 3)
+    got = rays.copy()
+    e.Intersect(got)
+    assert util.compare_hits(got, want) == ZERO
+    assert np.array_equal(e.IsOccluded(sh), want_bits), "occlusion"
     # statistics of a multi-chunk call = statistics of the same rays traced in one device launch
     import torch
     e.set_stats(True)

@@ -31,7 +31,7 @@ def context(device: int = 0):
 
 
 def set_option(key: str, value: int, device: int = 0) -> None:
-    """Tuning knob of the engine context (tbvh_set_option): trace_variant, small_t, d2h_mode, h2d_split, host_path."""
+    """Option of the engine context (tbvh_set_option): inst_idx_bits, small_t or build_mode; any other key raises TbvhError."""
     check(_lib.lib().tbvh_set_option(context(device), key.encode(), int(value)))
 
 

@@ -5,12 +5,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <vector>
-#include <thread>
-#include <atomic>
 #include <mutex>
-#include <condition_variable>
-#include <memory>
-#include <functional>
 #include <new>
 
 static thread_local char g_err[512] = "";
@@ -90,48 +85,6 @@ template <class F> static auto on_node( int node, F fn ) -> decltype( fn() )
 	return r;
 }
 
-// A few persistent host threads, bound to the CPUs of one NUMA node, that run fn( t, T ) in parallel and block the caller until
-// every slice is done (d2h_mode 2: hits scattered into the caller's strided ray records).
-struct HostPool
-{
-	HostPool( unsigned threads, int node ) : T( threads )
-	{
-		for (unsigned t = 0; t < T; t++) th.emplace_back( [this, t, node]()
-		{
-			cpu_set_t want;
-			if (node_cpus( node, &want )) sched_setaffinity( 0, sizeof( want ), &want );
-			uint64_t seen = 0;
-			for (;;)
-			{
-				std::unique_lock<std::mutex> lk( m );
-				cv_go.wait( lk, [&]() { return quit || gen != seen; } );
-				if (quit) return;
-				seen = gen;
-				lk.unlock();
-				job( t, T );
-				lk.lock();
-				if (++done == T) cv_done.notify_one();
-			}
-		} );
-	}
-	~HostPool() { { std::lock_guard<std::mutex> lk( m ); quit = true; } cv_go.notify_all(); for (auto& t : th) t.join(); }
-	template <class F> void run( F fn )
-	{
-		{ std::lock_guard<std::mutex> lk( m ); job = fn, done = 0, gen++; }
-		cv_go.notify_all();
-		std::unique_lock<std::mutex> lk( m );
-		cv_done.wait( lk, [&]() { return done == T; } );
-	}
-	unsigned T;
-	std::vector<std::thread> th;
-	std::mutex m;
-	std::condition_variable cv_go, cv_done;
-	std::function<void( unsigned, unsigned )> job;
-	uint64_t gen = 0;
-	unsigned done = 0;
-	bool quit = false;
-};
-
 extern "C" {
 
 const char* tbvh_last_error( void ) { return g_err; }
@@ -167,7 +120,6 @@ int tbvh_ctx_create( int device, tbvh_ctx* out )
 	tbvh_ctx c = new (std::nothrow) tbvh_ctx_t();
 	ARG_CHECK( c, "out of host memory" );
 	c->device = device;
-	c->numa_node = device_numa_node( device );
 	auto body = [&]() -> int
 	{
 		cudaDeviceProp prop;
@@ -177,61 +129,18 @@ int tbvh_ctx_create( int device, tbvh_ctx* out )
 		CUDA_TRY( cudaStreamCreateWithFlags( &c->s_in, cudaStreamNonBlocking ) );
 		CUDA_TRY( cudaStreamCreateWithFlags( &c->s_run, cudaStreamNonBlocking ) );
 		CUDA_TRY( cudaStreamCreateWithFlags( &c->s_out, cudaStreamNonBlocking ) );
-		for (int i = 0; i < 3; i++) CUDA_TRY( cudaStreamCreateWithFlags( &c->s_in_part[i], cudaStreamNonBlocking ) );
-		CUDA_TRY( cudaEventCreateWithFlags( &c->ev_fork, cudaEventDisableTiming ) );
 		for (int i = 0; i < TBVH_SLOTS; i++)
 		{
 			CUDA_TRY( cudaEventCreateWithFlags( &c->slot[i].in_done, cudaEventDisableTiming ) );
 			CUDA_TRY( cudaEventCreateWithFlags( &c->slot[i].run_done, cudaEventDisableTiming ) );
 			CUDA_TRY( cudaEventCreateWithFlags( &c->slot[i].out_done, cudaEventDisableTiming ) );
-			for (int p = 0; p < 3; p++) CUDA_TRY( cudaEventCreateWithFlags( &c->ev_part[i][p], cudaEventDisableTiming ) );
 		}
-		CUDA_TRY( cudaMalloc( &c->d_counters, TBVH_COUNTERS * 8 ) );
-		CUDA_TRY( cudaMemset( c->d_counters, 0, TBVH_COUNTERS * 8 ) );
 		return TBVH_OK;
 	};
 	const int rc = body();
 	if (rc != TBVH_OK) { tbvh_ctx_destroy( c ); return rc; }
-	const char* hp = getenv( "TBVH_HOST_PATH" );
-	c->host_path = hp && (!strcmp( hp, "zerocopy" ) || !strcmp( hp, "1" )) ? 1 : hp && !strcmp( hp, "2" ) ? 2 : 0;
-	const char* tv = getenv( "TBVH_TRACE_VARIANT" );
-	c->trace_variant = tv ? atoi( tv ) : 3; // octant switch: +5 % on camera / shadow rays, -3 % on diffuse (profiles/README.md)
-	const char* bc = getenv( "TBVH_BUILD_CTAS" );
-	if (bc) c->build_ctas = atoi( bc );
-	const char* bm = getenv( "TBVH_BUILD_MODE" );
-	if (bm) c->build_mode = atoi( bm ) ? 1 : 0;
-	const char* st = getenv( "TBVH_SMALL_T" );
-	c->small_t = st ? atoi( st ) : 128;
-	const char* hs = getenv( "TBVH_HQ_SMALL" );
-	if (hs) c->hq_small = atoi( hs );
-	const char* hc = getenv( "TBVH_HQ_CLUSTER" );
-	if (hc) c->hq_cluster = atoi( hc );
-	const char* dm = getenv( "TBVH_D2H_MODE" );
-	c->d2h_mode = dm ? atoi( dm ) : 1; // whole first cache lines back: +32 % in-place throughput with four GPUs on one socket, neutral with one (profiles/README.md)
-	if (c->d2h_mode < 0 || c->d2h_mode > 3) c->d2h_mode = 1;
-	const char* sp = getenv( "TBVH_H2D_SPLIT" );
-	c->h2d_split = sp ? atoi( sp ) : 1;
-	if (c->h2d_split < 1) c->h2d_split = 1;
-	if (c->h2d_split > 4) c->h2d_split = 4;
-	const char* stn = getenv( "TBVH_SCATTER_THREADS" );
-	if (stn && atoi( stn ) >= 1 && atoi( stn ) <= 64) c->scatter_threads = atoi( stn );
-	const char* cr = getenv( "TBVH_CHUNK_RAYS" );
-	if (cr && atol( cr ) >= 4096) c->chunk_rays = (size_t)atol( cr ) & ~(size_t)31;
 	*out = c;
 	return TBVH_OK;
-}
-
-static void free_slots( tbvh_ctx c )
-{
-	for (int i = 0; i < TBVH_SLOTS; i++)
-	{
-		if (c->slot[i].d_rays) cudaFree( c->slot[i].d_rays );
-		if (c->slot[i].d_hits) cudaFree( c->slot[i].d_hits );
-		if (c->slot[i].d_bits) cudaFree( c->slot[i].d_bits );
-		if (c->slot[i].h_hits) cudaFreeHost( c->slot[i].h_hits );
-		c->slot[i].d_rays = c->slot[i].d_hits = c->slot[i].d_bits = c->slot[i].h_hits = 0;
-	}
-	c->slot_rays = 0, c->slot_rec = 0;
 }
 
 int tbvh_ctx_destroy( tbvh_ctx c )
@@ -239,22 +148,19 @@ int tbvh_ctx_destroy( tbvh_ctx c )
 	if (!c) return TBVH_OK;
 	cudaSetDevice( c->device );
 	cudaDeviceSynchronize();
-	free_slots( c );
 	for (int i = 0; i < TBVH_SLOTS; i++)
 	{
+		if (c->slot[i].d_rays) cudaFree( c->slot[i].d_rays );
+		if (c->slot[i].d_hits) cudaFree( c->slot[i].d_hits );
+		if (c->slot[i].d_bits) cudaFree( c->slot[i].d_bits );
 		if (c->slot[i].in_done) cudaEventDestroy( c->slot[i].in_done );
 		if (c->slot[i].run_done) cudaEventDestroy( c->slot[i].run_done );
 		if (c->slot[i].out_done) cudaEventDestroy( c->slot[i].out_done );
-		for (int p = 0; p < 3; p++) if (c->ev_part[i][p]) cudaEventDestroy( c->ev_part[i][p] );
 	}
-	if (c->ev_fork) cudaEventDestroy( c->ev_fork );
-	for (int i = 0; i < 3; i++) if (c->s_in_part[i]) cudaStreamDestroy( c->s_in_part[i] );
 	if (c->s_in) cudaStreamDestroy( c->s_in );
 	if (c->s_run) cudaStreamDestroy( c->s_run );
 	if (c->s_out) cudaStreamDestroy( c->s_out );
 	if (c->stream) cudaStreamDestroy( c->stream );
-	if (c->d_counters) cudaFree( c->d_counters );
-	delete c->pool;
 	delete c;
 	return TBVH_OK;
 }
@@ -262,37 +168,9 @@ int tbvh_ctx_destroy( tbvh_ctx c )
 int tbvh_set_option( tbvh_ctx c, const char* key, int value )
 {
 	ARG_CHECK( c && key, "NULL argument" );
-	if (!strcmp( key, "trace_variant" )) c->trace_variant = value;
+	if (!strcmp( key, "inst_idx_bits" )) c->inst_idx_bits = value;
 	else if (!strcmp( key, "small_t" )) c->small_t = value;
-	else if (!strcmp( key, "small_mode" )) c->small_mode = value & 3;
 	else if (!strcmp( key, "build_mode" )) c->build_mode = value ? 1 : 0;
-	else if (!strcmp( key, "build_ctas" )) c->build_ctas = value < 0 ? 0 : value > 16 ? 16 : value;
-	else if (!strcmp( key, "inst_idx_bits" )) c->inst_idx_bits = value;
-	else if (!strcmp( key, "hq_small" )) c->hq_small = value;
-	else if (!strcmp( key, "hq_cluster" )) c->hq_cluster = value;
-	else if (!strcmp( key, "d2h_mode" )) c->d2h_mode = value >= 0 && value <= 3 ? value : 0;
-	else if (!strcmp( key, "scatter_threads" ))
-	{
-		ARG_CHECK( value >= 1 && value <= 64, "scatter_threads must be 1..64" );
-		std::lock_guard<std::mutex> lk( c->host_mutex );
-		delete c->pool;
-		c->pool = 0, c->scatter_threads = value;
-	}
-	else if (!strcmp( key, "h2d_split" )) c->h2d_split = value < 1 ? 1 : value > 4 ? 4 : value;
-	else if (!strcmp( key, "host_path" ))
-	{
-		std::lock_guard<std::mutex> lk( c->host_mutex );
-		c->host_path = value == 1 ? 1 : value == 2 ? 2 : 0;
-	}
-	else if (!strcmp( key, "chunk_rays" ))
-	{
-		ARG_CHECK( value >= 4096, "chunk_rays must be at least 4096" );
-		std::lock_guard<std::mutex> lk( c->host_mutex );
-		CUDA_TRY( cudaSetDevice( c->device ) );
-		CUDA_TRY( cudaDeviceSynchronize() );
-		free_slots( c );
-		c->chunk_rays = (size_t)value & ~(size_t)31;
-	}
 	else { tbvh_set_error( "tbvh_set_option: unknown key '%s'", key ); return TBVH_E_ARG; }
 	return TBVH_OK;
 }
@@ -972,88 +850,35 @@ int tbvh_copy_rays_to_device( const void* rays, uint32_t stride, uint64_t n, voi
 }
 
 // ---- host-buffer path ---------------------------------------------------------------------------------------------
-// tbvh_intersect / tbvh_intersect_packed / tbvh_occluded on HOST ray records.  Only bytes 0..63 of each record cross PCIe inbound
-// and only the 16-byte hit (or one bit) outbound.  The batch is cut into chunks that flow through TBVH_SLOTS stage buffers:
+// tbvh_intersect / tbvh_intersect_packed / tbvh_occluded on HOST ray records.  Only bytes 0..63 of each record cross PCIe inbound,
+// and outbound only what the call returns.  The batch is cut into chunks that flow through TBVH_SLOTS stage buffers:
 //
-//     s_in  : chunk k+1   host records --(2D copy of 64-byte rows, or a gather kernel through the pinned mapping)--> slot.d_rays
-//     s_run : chunk k     traversal kernel: slot.d_rays -> slot.d_hits (packed 16-byte hits) / slot.d_bits
-//     s_out : chunk k-1   slot.d_hits --(2D copy of 16-byte rows into Ray.hit, or one contiguous copy for the packed form)--> host
+//     s_in  : chunk k+1   host records --(2D copy of 64-byte rows)--> slot.d_rays
+//     s_run : chunk k     traversal kernel: hits into the staged records (in place, TLAS) or slot.d_hits (packed) / slot.d_bits
+//     s_out : chunk k-1   back to the host: bytes 0..63 of every record (in place), one contiguous copy (packed), 20-byte rows at
+//                         byte 44 (TLAS: instance + hit) or the occlusion words
 //
 // Each direction owns a stream, so the inbound copy engine never waits for an outbound copy queued ahead of it; events hand a
 // slot from stage to stage and back (out_done -> the next inbound copy into that slot).  One call at a time per context
 // (host_mutex): concurrent callers on one handle are serialised, as SURVEY 8(b) asks.
-__global__ void __launch_bounds__( 256 ) k_gather_rays( const float4* __restrict__ src, const uint32_t stride_f4, float4* __restrict__ dst, const uint64_t n )
-{
-	const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, r = t >> 2;
-	if (r < n) dst[t] = src[r * stride_f4 + (t & 3)];
-}
-
-__global__ void __launch_bounds__( 256 ) k_scatter_hits( const float4* __restrict__ src, float4* __restrict__ dst, const uint32_t stride_f4, const uint64_t n )
-{
-	const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if (r < n) dst[r * stride_f4 + 3] = src[r];
-}
-
-// device alias of a page-locked host pointer, or NULL when the memory is pageable
-static void* mapped_alias( const void* host )
-{
-	cudaPointerAttributes a;
-	if (cudaPointerGetAttributes( &a, host ) != cudaSuccess) { cudaGetLastError(); return 0; }
-	if (a.type != cudaMemoryTypeHost || !a.devicePointer) return 0;
-	return a.devicePointer;
-}
-
 static int ensure_slots( tbvh_ctx c )
 {
-	const size_t rec = c->host_path == 2 ? 128 : 64; // host_path 2 stages whole 128-byte records
-	if (c->slot_rays == c->chunk_rays && c->slot_rec >= rec) return TBVH_OK;
-	free_slots( c );
-	for (int i = 0; i < TBVH_SLOTS; i++)
+	// allocated once; a call that failed half-way leaves the buffers it got, and the next one completes the set
+	for (HostSlot& sl : c->slot)
 	{
-		CUDA_TRY( cudaMalloc( &c->slot[i].d_rays, c->chunk_rays * rec ) );
-		CUDA_TRY( cudaMalloc( &c->slot[i].d_hits, c->chunk_rays * 16 ) );
-		CUDA_TRY( cudaMalloc( &c->slot[i].d_bits, c->chunk_rays / 8 + 4 ) );
+		if (!sl.d_rays) CUDA_TRY( cudaMalloc( &sl.d_rays, (size_t)TBVH_CHUNK_RAYS * 64 ) );
+		if (!sl.d_hits) CUDA_TRY( cudaMalloc( &sl.d_hits, (size_t)TBVH_CHUNK_RAYS * 16 ) );
+		if (!sl.d_bits) CUDA_TRY( cudaMalloc( &sl.d_bits, TBVH_CHUNK_RAYS / 8 + 4 ) );
 	}
-	c->slot_rays = c->chunk_rays, c->slot_rec = rec;
 	return TBVH_OK;
 }
 
 // inbound stage of one chunk: on return s_in carries the copy and slot.in_done is recorded behind it
-static int stage_in( tbvh_ctx c, const int k, const uint64_t chunk, const char* h, const char* h_dev, const uint32_t stride, const uint64_t cnt, uint32_t* staged_stride )
+static int stage_in( tbvh_ctx c, const uint64_t chunk, const char* h, const uint32_t stride, const uint64_t cnt )
 {
-	HostSlot& sl = c->slot[k];
-	*staged_stride = 64;
+	HostSlot& sl = c->slot[chunk % TBVH_SLOTS];
 	if (chunk >= TBVH_SLOTS) CUDA_TRY( cudaStreamWaitEvent( c->s_in, sl.out_done, 0 ) ); // the slot's previous tenant has left the device
-	if (c->host_path == 2 && stride == 128 && c->slot_rec >= 128)
-	{
-		// whole records, one contiguous copy: twice the bytes, but large read requests (the 64-byte rows of the 2D copy keep the link
-		// at ~37 GB/s of useful data; a contiguous copy runs at ~54 GB/s, i.e. 27 GB/s useful - profiles/README.md has the numbers)
-		CUDA_TRY( cudaMemcpyAsync( sl.d_rays, h, cnt * 128, cudaMemcpyHostToDevice, c->s_in ) );
-		*staged_stride = 128;
-	}
-	else if (c->host_path == 1 && h_dev && (stride & 15) == 0)
-	{
-		const uint64_t threads = cnt * 4;
-		k_gather_rays<<<(uint32_t)((threads + 255) / 256), 256, 0, c->s_in>>>( (const float4*)h_dev, stride / 16, (float4*)sl.d_rays, cnt );
-		LAUNCHED();
-	}
-	else if (c->h2d_split > 1 && cnt >= 4096)
-	{
-		// rows of the chunk spread over several streams so more than one copy engine pulls them; s_in joins the parts
-		const int parts = c->h2d_split;
-		const uint64_t per = ((cnt + parts - 1) / parts + 31) & ~31ull;
-		CUDA_TRY( cudaEventRecord( c->ev_fork, c->s_in ) );
-		for (int p = 0; p < parts; p++)
-		{
-			const uint64_t a = per * p, e = a + per < cnt ? a + per : cnt;
-			if (a >= e) break;
-			cudaStream_t ps = p == 0 ? c->s_in : c->s_in_part[p - 1];
-			if (p) CUDA_TRY( cudaStreamWaitEvent( ps, c->ev_fork, 0 ) );
-			CUDA_TRY( cudaMemcpy2DAsync( (char*)sl.d_rays + a * 64, 64, h + a * stride, stride, 64, e - a, cudaMemcpyHostToDevice, ps ) );
-			if (p) { CUDA_TRY( cudaEventRecord( c->ev_part[k][p - 1], ps ) ); CUDA_TRY( cudaStreamWaitEvent( c->s_in, c->ev_part[k][p - 1], 0 ) ); }
-		}
-	}
-	else CUDA_TRY( cudaMemcpy2DAsync( sl.d_rays, 64, h, stride, 64, cnt, cudaMemcpyHostToDevice, c->s_in ) );
+	CUDA_TRY( cudaMemcpy2DAsync( sl.d_rays, 64, h, stride, 64, cnt, cudaMemcpyHostToDevice, c->s_in ) );
 	CUDA_TRY( cudaEventRecord( sl.in_done, c->s_in ) );
 	CUDA_TRY( cudaStreamWaitEvent( c->s_run, sl.in_done, 0 ) );
 	return TBVH_OK;
@@ -1081,74 +906,32 @@ static int intersect_host( tbvh_bvh b, int layout, void* rays, uint32_t stride, 
 		if (packed_hits) { tbvh_set_error( "tbvh_intersect_packed: TLAS hits carry the instance and are returned in the ray records" ); return TBVH_E_UNSUPPORTED; }
 		TRY( tlas_check( b, layout ) );
 	}
-	char* dev_alias = (char*)mapped_alias( rays );
-	const bool scatter = !packed_hits && !tlas && c->d2h_mode == 3 && dev_alias && (stride & 15) == 0;
-	// d2h_mode 1: the kernel writes the hit into the staged record and bytes 0..63 of every record - exactly its first cache line - travel
-	// back, so the host receives FULL-line writes (no read-for-ownership of a partially written line); bytes 0..47 return unchanged
-	const bool full_line = !packed_hits && !tlas && c->d2h_mode == 1 && stride >= 64;
-	// d2h_mode 2: the hits leave the device packed (one contiguous copy per chunk) into page-locked staging, and a few host threads on
-	// the device's NUMA node write them into the strided records while later chunks are in flight
-	const bool host_scatter = !packed_hits && !tlas && c->d2h_mode == 2 && n >= 65536;
-	if (host_scatter)
-	{
-		for (int i = 0; i < TBVH_SLOTS; i++) if (!c->slot[i].h_hits)
-		{
-			const cudaError_t e = on_node( c->numa_node, [&]() { return cudaHostAlloc( &c->slot[i].h_hits, c->chunk_rays * 16, cudaHostAllocDefault ); } );
-			if (e != cudaSuccess) { tbvh_set_error( "host staging: %s", cudaGetErrorString( e ) ); return TBVH_E_CUDA; }
-		}
-		if (!c->pool) c->pool = new HostPool( (unsigned)c->scatter_threads, c->numa_node );
-	}
-	// hits of chunk `ch` (already on their way to slot staging) -> the caller's records
-	auto scatter_chunk = [&]( const uint64_t ch ) -> int
-	{
-		HostSlot& sl = c->slot[ch % TBVH_SLOTS];
-		CUDA_TRY( cudaEventSynchronize( sl.out_done ) );
-		const uint64_t off = ch * c->chunk_rays, cnt = n - off < c->chunk_rays ? n - off : c->chunk_rays;
-		char* dst = (char*)rays + off * stride + 48;
-		const char* src = (const char*)sl.h_hits;
-		c->pool->run( [=]( unsigned t, unsigned T )
-		{
-			const uint64_t per = (cnt + T - 1) / T, a = per * t, e = a + per < cnt ? a + per : cnt;
-			for (uint64_t i = a; i < e; i++) memcpy( dst + i * stride, src + i * 16, 16 );
-		} );
-		return TBVH_OK;
-	};
 	uint64_t chunk = 0;
 	int rc = TBVH_OK;
-	for (uint64_t off = 0; off < n && rc == TBVH_OK; off += c->chunk_rays, chunk++)
+	for (uint64_t off = 0; off < n && rc == TBVH_OK; off += TBVH_CHUNK_RAYS, chunk++)
 	{
-		const int k = (int)(chunk % TBVH_SLOTS);
-		HostSlot& sl = c->slot[k];
-		const uint64_t cnt = n - off < c->chunk_rays ? n - off : c->chunk_rays;
+		HostSlot& sl = c->slot[chunk % TBVH_SLOTS];
+		const uint64_t cnt = n - off < TBVH_CHUNK_RAYS ? n - off : TBVH_CHUNK_RAYS;
 		char* h = (char*)rays + off * stride;
-		char* hd = dev_alias ? dev_alias + off * stride : 0;
 		auto body = [&]() -> int
 		{
-			if (host_scatter && chunk >= TBVH_SLOTS) TRY( scatter_chunk( chunk - TBVH_SLOTS ) ); // frees this slot's staging
-			uint32_t ss = 64;
-			TRY( stage_in( c, k, chunk, h, hd, stride, cnt, &ss ) );
-			if (tlas) TRY( tlas_trace_launch( b, layout, sl.d_rays, ss, 0, cnt, false, c->s_run ) );  // hit + instance written into the staged records
-			else if (full_line) TRY( trace_dispatch( b, layout, sl.d_rays, ss, (char*)sl.d_rays + 48, ss, 0, cnt, false, c->s_run ) );
-			else TRY( trace_dispatch( b, layout, sl.d_rays, ss, sl.d_hits, 16, 0, cnt, false, c->s_run ) );
+			TRY( stage_in( c, chunk, h, stride, cnt ) );
+			// in place, the kernel writes the hit into the staged record and bytes 0..63 of every record - exactly its first cache line -
+			// travel back, so the host receives FULL-line writes (no read-for-ownership of a partially written line); bytes 0..47 return
+			// unchanged.  A TLAS writes hit + instance into the staged records as well.
+			if (tlas) TRY( tlas_trace_launch( b, layout, sl.d_rays, 64, 0, cnt, false, c->s_run ) );
+			else if (packed_hits) TRY( trace_dispatch( b, layout, sl.d_rays, 64, sl.d_hits, 16, 0, cnt, false, c->s_run ) );
+			else TRY( trace_dispatch( b, layout, sl.d_rays, 64, (char*)sl.d_rays + 48, 64, 0, cnt, false, c->s_run ) );
 			CUDA_TRY( cudaEventRecord( sl.run_done, c->s_run ) );
 			CUDA_TRY( cudaStreamWaitEvent( c->s_out, sl.run_done, 0 ) );
-			if (tlas) CUDA_TRY( cudaMemcpy2DAsync( h + 44, stride, (char*)sl.d_rays + 44, ss, 20, cnt, cudaMemcpyDeviceToHost, c->s_out ) );
+			if (tlas) CUDA_TRY( cudaMemcpy2DAsync( h + 44, stride, (char*)sl.d_rays + 44, 64, 20, cnt, cudaMemcpyDeviceToHost, c->s_out ) );
 			else if (packed_hits) CUDA_TRY( cudaMemcpyAsync( (char*)packed_hits + off * 16, sl.d_hits, cnt * 16, cudaMemcpyDeviceToHost, c->s_out ) );
-			else if (host_scatter) CUDA_TRY( cudaMemcpyAsync( sl.h_hits, sl.d_hits, cnt * 16, cudaMemcpyDeviceToHost, c->s_out ) );
-			else if (full_line) CUDA_TRY( cudaMemcpy2DAsync( h, stride, sl.d_rays, ss, 64, cnt, cudaMemcpyDeviceToHost, c->s_out ) );
-			else if (scatter)
-			{
-				k_scatter_hits<<<(uint32_t)((cnt + 255) / 256), 256, 0, c->s_out>>>( (const float4*)sl.d_hits, (float4*)hd, stride / 16, cnt );
-				LAUNCHED();
-			}
-			else CUDA_TRY( cudaMemcpy2DAsync( h + 48, stride, sl.d_hits, 16, 16, cnt, cudaMemcpyDeviceToHost, c->s_out ) );
+			else CUDA_TRY( cudaMemcpy2DAsync( h, stride, sl.d_rays, 64, 64, cnt, cudaMemcpyDeviceToHost, c->s_out ) );
 			CUDA_TRY( cudaEventRecord( sl.out_done, c->s_out ) );
 			return TBVH_OK;
 		};
 		rc = body();
 	}
-	if (host_scatter && rc == TBVH_OK)
-		for (uint64_t ch = chunk > TBVH_SLOTS ? chunk - TBVH_SLOTS : 0; ch < chunk && rc == TBVH_OK; ch++) rc = scatter_chunk( ch );
 	const int rd = drain( c ); // also after an error: nothing of this call may still be in flight when the mutex is released
 	return rc != TBVH_OK ? rc : rd;
 }
@@ -1170,24 +953,21 @@ int tbvh_occluded( tbvh_bvh b, int layout, const void* rays, uint32_t stride, ui
 	TRY( ensure_slots( c ) );
 	if (b->stats) CUDA_TRY( cudaMemset( b->d_stats, 0, 32 ) );
 	if (b->d_inst) TRY( tlas_check( b, layout ) );
-	const char* dev_alias = (const char*)mapped_alias( rays );
 	uint64_t chunk = 0;
 	int rc = TBVH_OK;
-	for (uint64_t off = 0; off < n && rc == TBVH_OK; off += c->chunk_rays, chunk++)
+	for (uint64_t off = 0; off < n && rc == TBVH_OK; off += TBVH_CHUNK_RAYS, chunk++)
 	{
-		const int k = (int)(chunk % TBVH_SLOTS);
-		HostSlot& sl = c->slot[k];
-		const uint64_t cnt = n - off < c->chunk_rays ? n - off : c->chunk_rays;
+		HostSlot& sl = c->slot[chunk % TBVH_SLOTS];
+		const uint64_t cnt = n - off < TBVH_CHUNK_RAYS ? n - off : TBVH_CHUNK_RAYS;
 		const char* h = (const char*)rays + off * stride;
 		auto body = [&]() -> int
 		{
-			uint32_t ss = 64;
-			TRY( stage_in( c, k, chunk, h, dev_alias ? dev_alias + off * stride : 0, stride, cnt, &ss ) );
-			if (b->d_inst) TRY( tlas_trace_launch( b, layout, sl.d_rays, ss, (uint32_t*)sl.d_bits, cnt, true, c->s_run ) );
-			else TRY( trace_dispatch( b, layout, sl.d_rays, ss, 0, 0, (uint32_t*)sl.d_bits, cnt, true, c->s_run ) );
+			TRY( stage_in( c, chunk, h, stride, cnt ) );
+			if (b->d_inst) TRY( tlas_trace_launch( b, layout, sl.d_rays, 64, (uint32_t*)sl.d_bits, cnt, true, c->s_run ) );
+			else TRY( trace_dispatch( b, layout, sl.d_rays, 64, 0, 0, (uint32_t*)sl.d_bits, cnt, true, c->s_run ) );
 			CUDA_TRY( cudaEventRecord( sl.run_done, c->s_run ) );
 			CUDA_TRY( cudaStreamWaitEvent( c->s_out, sl.run_done, 0 ) );
-			CUDA_TRY( cudaMemcpyAsync( bits + off / 32, sl.d_bits, ((cnt + 31) / 32) * 4, cudaMemcpyDeviceToHost, c->s_out ) ); // chunk_rays is a multiple of 32
+			CUDA_TRY( cudaMemcpyAsync( bits + off / 32, sl.d_bits, ((cnt + 31) / 32) * 4, cudaMemcpyDeviceToHost, c->s_out ) ); // TBVH_CHUNK_RAYS is a multiple of 32
 			CUDA_TRY( cudaEventRecord( sl.out_done, c->s_out ) );
 			return TBVH_OK;
 		};

@@ -34,8 +34,10 @@ namespace cg = cooperative_groups;
 namespace
 {
 #define HQBINS 8
-#define HQ_SMALL_MAX 256      // switch point CTA/cluster per node -> warp per subtree (run-time value hq_small <= this)
-#define HQ_MAX_CLUSTER 16
+#define HQ_SMALL 16            // switch point CTA/cluster per node -> warp per subtree: nodes of at most this many fragments
+#define HQ_MAX_CLUSTER 16      // largest thread-block cluster a node of the level phase gets
+#define HQ_CTA_FRAGS 512       // cluster sizing: about this many fragments per CTA of the level's largest node
+#define HQ_CTA_CAP 16          // cluster sizing: 2 x (CTAs of the level) <= this x SMs, i.e. at most 8 CTAs per SM in flight
 #define HQ_MLP 4               // independent index -> fragment load chains per thread in the binning loops
 #define HQ_E 8                 // consecutive fragments per thread and scan tile of the partition passes (8 * 4096 fits the 16-bit packed counters)
 #define HQ_BIG_THREADS 256
@@ -68,7 +70,7 @@ struct HQArgs
 	float4* tmp_nodes; uint32_t* parent; uint32_t* sub_int; uint32_t* sub_prims; uint32_t* arrive;
 	HQTask* lvl[2]; HQTask* small;
 	HQCounters* ctr;
-	uint32_t n, idx_cap, node_cap, lvl_cap, small_t, profile;
+	uint32_t n, idx_cap, node_cap, lvl_cap, profile;
 	float c_trav, c_int;
 };
 
@@ -980,13 +982,13 @@ __global__ void k_hq_root( HQArgs A )
 	c->root_area = half_area3( ex, ey, ez );
 	c->min_dim[0] = __fmul_rn( ex, 1e-7f ), c->min_dim[1] = __fmul_rn( ey, 1e-7f ), c->min_dim[2] = __fmul_rn( ez, 1e-7f );
 	HQTask t = { 0u, 0u, A.idx_cap, 0u };
-	if (A.n > A.small_t) A.lvl[0][0] = t, c->next_big = 1, c->next_max = A.n; else A.small[0] = t, c->small_roots = 1;
+	if (A.n > HQ_SMALL) A.lvl[0][0] = t, c->next_big = 1, c->next_max = A.n; else A.small[0] = t, c->small_roots = 1;
 }
 
 __device__ __forceinline__ void hq_enqueue( const HQArgs& A, HQTask* next, const HQTask c )
 {
 	const uint32_t cnt = __float_as_uint( A.tmp_nodes[(size_t)c.node * 2 + 1].w );
-	if (cnt > A.small_t)
+	if (cnt > HQ_SMALL)
 	{
 		atomicMax( &A.ctr->next_max, cnt );
 		const uint32_t k = atomicAdd( &A.ctr->next_big, 1u );
@@ -1104,11 +1106,7 @@ int build_hq_launch( tbvh_bvh b, float c_trav, float c_int )
 	HQArgs A = {};
 	A.verts = b->d_verts, A.n = n, A.c_trav = c_trav, A.c_int = c_int;
 	A.idx_cap = n + slack, A.node_cap = 3 * n + 2;
-	{
-		const int t = b->ctx->hq_small;
-		A.small_t = (uint32_t)(t < 8 ? 8 : t > HQ_SMALL_MAX ? HQ_SMALL_MAX : t);
-	}
-	A.lvl_cap = A.idx_cap / A.small_t + 2;
+	A.lvl_cap = A.idx_cap / HQ_SMALL + 2;
 	{ const char* e = getenv( "TBVH_HQ_PROFILE" ); A.profile = e ? (uint32_t)atoi( e ) : 0u; }
 	HQCounters* h_ctr = 0;
 	cudaEvent_t e0 = 0, e1 = 0;
@@ -1134,18 +1132,15 @@ int build_hq_launch( tbvh_bvh b, float c_trav, float c_int )
 		k_hq_init<<<1, 1, 0, s>>>( A ); LAUNCHED();
 		k_hq_fragments<<<(n + 255) / 256, 256, 0, s>>>( A ); LAUNCHED();
 		k_hq_root<<<1, 1, 0, s>>>( A ); LAUNCHED();
-		uint32_t num = n > A.small_t ? 1 : 0, level = 0, max_count = n;
-		uint32_t max_cluster = (uint32_t)(b->ctx->hq_cluster < 1 ? 1 : b->ctx->hq_cluster > HQ_MAX_CLUSTER ? HQ_MAX_CLUSTER : b->ctx->hq_cluster);
-		// tuning knobs of the cluster sizing rule (defaults measured on B200, profiles/README.md)
-		const char* env_cf = getenv( "TBVH_HQ_CTA_FRAGS" ); const char* env_cc = getenv( "TBVH_HQ_CTA_CAP" );
-		const size_t cta_frags = env_cf && atoi( env_cf ) > 0 ? (size_t)atoi( env_cf ) : 512, cta_cap = env_cc && atoi( env_cc ) > 0 ? (size_t)atoi( env_cc ) : 16;
-		if (max_cluster > 8) CUDA_TRY( cudaFuncSetAttribute( k_hq_level, cudaFuncAttributeNonPortableClusterSizeAllowed, 1 ) );
+		uint32_t num = n > HQ_SMALL ? 1 : 0, level = 0, max_count = n, max_cluster = HQ_MAX_CLUSTER;
+		CUDA_TRY( cudaFuncSetAttribute( k_hq_level, cudaFuncAttributeNonPortableClusterSizeAllowed, 1 ) ); // clusters of more than 8 CTAs
 		while (num)
 		{
 			CUDA_TRY( cudaMemsetAsync( &A.ctr->next_big, 0, 8, s ) ); // next_big + next_max
-			// cluster size: enough CTAs for the largest node of the level (about 512 fragments per CTA), at most 8 CTAs per SM in flight
+			// cluster size: enough CTAs for the largest node of the level, at most 8 CTAs per SM in flight (constants measured on B200,
+			// profiles/README.md)
 			uint32_t nct = 1;
-			while (nct < max_cluster && (size_t)nct * cta_frags < max_count && (size_t)num * nct * 2 <= (size_t)b->ctx->sm_count * cta_cap) nct <<= 1;
+			while (nct < max_cluster && (size_t)nct * HQ_CTA_FRAGS < max_count && (size_t)num * nct * 2 <= (size_t)b->ctx->sm_count * HQ_CTA_CAP) nct <<= 1;
 			cudaLaunchConfig_t cfg = {};
 			cudaLaunchAttribute attr[1];
 			cfg.gridDim = dim3( num * nct ), cfg.blockDim = dim3( HQ_BIG_THREADS ), cfg.dynamicSmemBytes = 0, cfg.stream = s;

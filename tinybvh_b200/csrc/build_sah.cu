@@ -24,6 +24,7 @@
 #define BINS 8
 #define SMALL_T 128          // capacity of the warp kernel: subtrees of at most this many primitives (run-time switch point <= this)
 #define CHUNK 256            // primitives per CTA in the large phase
+#define BUILD_CTAS_PER_SM 4  // resident CTAs per SM of the persistent large phase (k_large_phase)
 #define BIN_WORDS 168        // 3 axes x 8 bins x (3 min keys, 3 max keys, count)
 #define BIN_STRIDE 192       // + 3 x 8 counts of the PARTITION's own bin function (BuildAVX flavour, see bin_part_avx)
 __device__ __forceinline__ uint32_t bin_init_word( const uint32_t k ) { return (k < BIN_WORDS && (k % 7) < 3) ? 0xffffffffu : 0u; }
@@ -61,7 +62,7 @@ struct BuildArgs
 	Counters* ctr;
 	uint32_t n;
 	uint32_t flavour;        // 0 = BVH::Build (scalar reference builder), 1 = BVH::BuildAVX (what BuildDefault runs on x86)
-	uint32_t small_t;        // runtime switch point large phase -> warp subtrees (<= SMALL_T; env TBVH_SMALL_T for tuning)
+	uint32_t small_t;        // runtime switch point large phase -> warp subtrees (<= SMALL_T; the context's small_t)
 	uint32_t level0;         // persistent large phase: the level it starts at (the launch-per-stage path may have run the first ones)
 	float c_trav, c_int;
 };
@@ -723,10 +724,9 @@ __global__ void __launch_bounds__( CHUNK ) k_large_phase( BuildArgs A )
 // ---------------------------------------------------------------------------------------------- small subtrees
 
 #define SMALL_WARPS 8
-template <bool FRAGS> struct SmallSmemT
+struct SmallSmem
 {
 	uint32_t gid[SMALL_T];            // global primitive index of each local slot
-	float fmn[FRAGS ? SMALL_T : 1][3], fmx[FRAGS ? SMALL_T : 1][3]; // FRAGS: the subtree's fragment boxes, staged once
 	uint16_t idx[2][SMALL_T];         // ping-pong order of local slots
 	uint16_t bid[SMALL_T];
 	uint16_t posbl[SMALL_T];
@@ -735,13 +735,8 @@ template <bool FRAGS> struct SmallSmemT
 	uint32_t st_tmp[12]; uint32_t st_rng[12]; uint32_t st_db[12]; // stack: tmp node, lo | n << 16, depth | buf << 16
 };
 
-// FRAGS: stage the subtree's fragment boxes in shared memory (no global gathers per level, fewer resident warps).
-// AGG:   warp-aggregated bin updates for batches of a node with >= 64 primitives (small nodes use plain shared atomics:
-//        with a handful of active lanes the match/redux sequence costs more than the conflicts it removes).
-template <bool FRAGS, bool AGG>
 __global__ void __launch_bounds__( SMALL_WARPS * 32 ) k_build_small( BuildArgs A, const uint32_t num_roots )
 {
-	typedef SmallSmemT<FRAGS> SmallSmem;
 	// One warp builds a whole subtree of <= SMALL_T primitives: the reference's loop (:2347-2445) with the primitives
 	// of the current node spread over the lanes.  The smaller child is continued, the larger pushed, so the stack
 	// stays below log2(SMALL_T)+2 entries; order of work does not matter because numbering is fixed afterwards.
@@ -752,16 +747,7 @@ __global__ void __launch_bounds__( SMALL_WARPS * 32 ) k_build_small( BuildArgs A
 	SmallSmem& S = S_all[wid];
 	const SmallRoot root = A.small[r];
 	const uint32_t* src = A.idx[root.depth_buf >> 16];
-	for (uint32_t k = lane; k < root.count; k += 32)
-	{
-		const uint32_t fi = src[root.first + k];
-		S.gid[k] = fi, S.idx[0][k] = (uint16_t)k;
-		if (FRAGS)
-		{
-			const float4 mn = __ldg( A.frag_min + fi ), mx = __ldg( A.frag_max + fi );
-			S.fmn[k][0] = mn.x, S.fmn[k][1] = mn.y, S.fmn[k][2] = mn.z, S.fmx[k][0] = mx.x, S.fmx[k][1] = mx.y, S.fmx[k][2] = mx.z;
-		}
-	}
+	for (uint32_t k = lane; k < root.count; k += 32) S.gid[k] = src[root.first + k], S.idx[0][k] = (uint16_t)k;
 	const float4 rmin = A.tmp_nodes[0], rmax = A.tmp_nodes[1];
 	const float mdf = A.flavour ? 1e-7f : 1e-20f; // minDim (:2346 / :6555)
 	const float3 min_dim = make_float3( __fmul_rn( __fsub_rn( rmax.x, rmin.x ), mdf ), __fmul_rn( __fsub_rn( rmax.y, rmin.y ), mdf ), __fmul_rn( __fsub_rn( rmax.z, rmin.z ), mdf ) );
@@ -777,50 +763,31 @@ __global__ void __launch_bounds__( SMALL_WARPS * 32 ) k_build_small( BuildArgs A
 		const float ex_ = __fsub_rn( nmax.x, nmin.x ), ey_ = __fsub_rn( nmax.y, nmin.y ), ez_ = __fsub_rn( nmax.z, nmin.z );
 		const float rpx = A.flavour ? rpd_avx( ex_ ) : __fdiv_rn( (float)BINS, ex_ ), rpy = A.flavour ? rpd_avx( ey_ ) : __fdiv_rn( (float)BINS, ey_ ), rpz = A.flavour ? rpd_avx( ez_ ) : __fdiv_rn( (float)BINS, ez_ );
 		const float mx2 = __fmul_rn( nmin.x, 2.0f ), my2 = __fmul_rn( nmin.y, 2.0f ), mz2 = __fmul_rn( nmin.z, 2.0f );
-		for (uint32_t base = 0; base < n; base += 32) // whole warp iterates together: the aggregated update votes
+		for (uint32_t k = lane; k < n; k += 32)
 		{
-			const uint32_t k = base + lane;
-			const bool valid = k < n;
-			uint32_t b3[3] = { 0, 0, 0 }, kmn[3] = { 0xffffffffu, 0xffffffffu, 0xffffffffu }, kmx[3] = { 0, 0, 0 };
-			if (valid)
+			const uint32_t sl = S.idx[buf][lo + k];
+			const float4 mn = __ldg( A.frag_min + S.gid[sl] ), mx = __ldg( A.frag_max + S.gid[sl] );
+			uint32_t b3[3];
+			if (A.flavour)
 			{
-				const uint32_t sl = S.idx[buf][lo + k];
-				float mnx, mny, mnz, mxx, mxy, mxz;
-				if (FRAGS) mnx = S.fmn[sl][0], mny = S.fmn[sl][1], mnz = S.fmn[sl][2], mxx = S.fmx[sl][0], mxy = S.fmx[sl][1], mxz = S.fmx[sl][2];
-				else
-				{
-					const float4 mn = __ldg( A.frag_min + S.gid[sl] ), mx = __ldg( A.frag_max + S.gid[sl] );
-					mnx = mn.x, mny = mn.y, mnz = mn.z, mxx = mx.x, mxy = mx.y, mxz = mx.z;
-				}
-				if (A.flavour)
-				{
-					b3[0] = bin_of_avx( mnx, mxx, mx2, rpx ), b3[1] = bin_of_avx( mny, mxy, my2, rpy ), b3[2] = bin_of_avx( mnz, mxz, mz2, rpz );
-					const uint32_t p0 = bin_part_avx( mnx, mxx, mx2, rpx ), p1 = bin_part_avx( mny, mxy, my2, rpy ), p2 = bin_part_avx( mnz, mxz, mz2, rpz );
-					S.bid[lo + k] = (uint16_t)(p0 | (p1 << 3) | (p2 << 6));
-					atomicAdd( S.bins + BIN_WORDS + p0, 1u ), atomicAdd( S.bins + BIN_WORDS + BINS + p1, 1u ), atomicAdd( S.bins + BIN_WORDS + 2 * BINS + p2, 1u );
-				}
-				else
-				{
-					b3[0] = bin_of( mnx, mxx, nmin.x, rpx ), b3[1] = bin_of( mny, mxy, nmin.y, rpy ), b3[2] = bin_of( mnz, mxz, nmin.z, rpz );
-					S.bid[lo + k] = (uint16_t)(b3[0] | (b3[1] << 3) | (b3[2] << 6));
-				}
-				kmn[0] = f2key( mnx ), kmn[1] = f2key( mny ), kmn[2] = f2key( mnz ), kmx[0] = f2key( mxx ), kmx[1] = f2key( mxy ), kmx[2] = f2key( mxz );
+				b3[0] = bin_of_avx( mn.x, mx.x, mx2, rpx ), b3[1] = bin_of_avx( mn.y, mx.y, my2, rpy ), b3[2] = bin_of_avx( mn.z, mx.z, mz2, rpz );
+				const uint32_t p0 = bin_part_avx( mn.x, mx.x, mx2, rpx ), p1 = bin_part_avx( mn.y, mx.y, my2, rpy ), p2 = bin_part_avx( mn.z, mx.z, mz2, rpz );
+				S.bid[lo + k] = (uint16_t)(p0 | (p1 << 3) | (p2 << 6));
+				atomicAdd( S.bins + BIN_WORDS + p0, 1u ), atomicAdd( S.bins + BIN_WORDS + BINS + p1, 1u ), atomicAdd( S.bins + BIN_WORDS + 2 * BINS + p2, 1u );
 			}
-			if (AGG && n >= 64)
+			else
 			{
-				#pragma unroll
-				for (int a = 0; a < 3; a++) bin_update_aggregated( S.bins + a * BINS * 7, valid, b3[a], kmn[0], kmn[1], kmn[2], kmx[0], kmx[1], kmx[2] );
+				b3[0] = bin_of( mn.x, mx.x, nmin.x, rpx ), b3[1] = bin_of( mn.y, mx.y, nmin.y, rpy ), b3[2] = bin_of( mn.z, mx.z, nmin.z, rpz );
+				S.bid[lo + k] = (uint16_t)(b3[0] | (b3[1] << 3) | (b3[2] << 6));
 			}
-			else if (valid)
+			const uint32_t kmn[3] = { f2key( mn.x ), f2key( mn.y ), f2key( mn.z ) }, kmx[3] = { f2key( mx.x ), f2key( mx.y ), f2key( mx.z ) };
+			#pragma unroll
+			for (int a = 0; a < 3; a++)
 			{
-				#pragma unroll
-				for (int a = 0; a < 3; a++)
-				{
-					uint32_t* w = S.bins + (a * BINS + b3[a]) * 7;
-					atomicMin( w + 0, kmn[0] ), atomicMin( w + 1, kmn[1] ), atomicMin( w + 2, kmn[2] );
-					atomicMax( w + 3, kmx[0] ), atomicMax( w + 4, kmx[1] ), atomicMax( w + 5, kmx[2] );
-					atomicAdd( w + 6, 1u );
-				}
+				uint32_t* w = S.bins + (a * BINS + b3[a]) * 7;
+				atomicMin( w + 0, kmn[0] ), atomicMin( w + 1, kmn[1] ), atomicMin( w + 2, kmn[2] );
+				atomicMax( w + 3, kmx[0] ), atomicMax( w + 4, kmx[1] ), atomicMax( w + 5, kmx[2] );
+				atomicAdd( w + 6, 1u );
 			}
 		}
 		__syncwarp();
@@ -1035,8 +1002,7 @@ int build_sah_launch( tbvh_bvh b, float c_trav, float c_int, int flavour )
 		if (num && b->ctx->build_mode == 0)
 		{
 			CUDA_TRY( cudaOccupancyMaxActiveBlocksPerMultiprocessor( &per_sm, k_large_phase, CHUNK, 0 ) );
-			const int want = b->ctx->build_ctas > 0 ? b->ctx->build_ctas : 4;
-			if (per_sm > want) per_sm = want;
+			if (per_sm > BUILD_CTAS_PER_SM) per_sm = BUILD_CTAS_PER_SM;
 			pgrid = (uint32_t)(per_sm > 0 ? per_sm * b->ctx->sm_count : 0);
 		}
 		const uint32_t persist_chunks = pgrid * 3;
@@ -1090,11 +1056,7 @@ int build_sah_launch( tbvh_bvh b, float c_trav, float c_int, int flavour )
 		const uint32_t roots = h_ctr->small_roots;
 		if (roots)
 		{
-			const uint32_t g = (roots + SMALL_WARPS - 1) / SMALL_WARPS, mode = (uint32_t)b->ctx->small_mode;
-			if (mode == 0) k_build_small<false, false><<<g, SMALL_WARPS * 32, 0, s>>>( A, roots );
-			else if (mode == 1) k_build_small<true, false><<<g, SMALL_WARPS * 32, 0, s>>>( A, roots );
-			else if (mode == 2) k_build_small<false, true><<<g, SMALL_WARPS * 32, 0, s>>>( A, roots );
-			else k_build_small<true, true><<<g, SMALL_WARPS * 32, 0, s>>>( A, roots );
+			k_build_small<<<(roots + SMALL_WARPS - 1) / SMALL_WARPS, SMALL_WARPS * 32, 0, s>>>( A, roots );
 			LAUNCHED();
 		}
 		CUDA_TRY( cudaMemcpyAsync( h_ctr, A.ctr, sizeof( Counters ), cudaMemcpyDeviceToHost, s ) );

@@ -25,48 +25,25 @@ struct HostSlot
 	void* d_rays = 0;                // chunk of 64-byte device records
 	void* d_hits = 0;                // packed 16-byte hits of the chunk
 	void* d_bits = 0;                // occlusion words of the chunk
-	void* h_hits = 0;                // page-locked staging for the chunk's packed hits (d2h_mode 2: scattered into the records by host threads)
 	cudaEvent_t in_done = 0, run_done = 0, out_done = 0;
 };
 #define TBVH_SLOTS 4
+#define TBVH_CHUNK_RAYS (1u << 19)   // rays per pipeline chunk (32 MiB of device records; 2^18 and 2^20 measured no better, profiles/README.md)
 
 struct tbvh_ctx_t
 {
 	int device = 0;
 	int sm_count = 148;
-	int numa_node = -1;              // host NUMA node the device hangs off (-1 = unknown)
 	cudaStream_t stream = 0;         // engine stream (builds, uploads, conversions)
 	// host-buffer pipeline: inbound copies, traversal and outbound copies each own a stream, so chunk k+1 flows in while chunk k
 	// is traced and the hits of chunk k-1 flow out; the slots are handed round-robin and recycled through events
 	std::mutex host_mutex;           // host batch calls on one context are serialised (SURVEY 8(b): thread-safe per handle)
 	cudaStream_t s_in = 0, s_run = 0, s_out = 0;
-	cudaStream_t s_in_part[3] = { 0, 0, 0 }; // extra inbound streams when h2d_split > 1
-	cudaEvent_t ev_part[TBVH_SLOTS][3] = {};
-	cudaEvent_t ev_fork = 0;
-	HostSlot slot[TBVH_SLOTS];
-	size_t chunk_rays = 1u << 19;    // rays per chunk (32 MiB of device records)
-	size_t slot_rays = 0;            // capacity the slots were allocated for
-	size_t slot_rec = 0;             // bytes per staged ray record the slots were allocated for (64, or 128 under host_path 2)
-	int host_path = 0;               // inbound: 0 = copy engine (cudaMemcpy2DAsync of 64-byte rows), 1 = gather kernel through the pinned mapping, 2 = whole 128-byte records in one contiguous copy
-	int h2d_split = 1;               // inbound 2D copy of a chunk split over this many streams (copy engines)
-	int d2h_mode = 1;                // in-place hits: 1 = bytes 0..63 of every record return (full cache lines, the default), 0 = 2D copy of 16-byte rows,
-	                                 // 2 = packed copy + host threads scatter, 3 = scatter kernel through the pinned mapping
-	int scatter_threads = 8;         // d2h_mode 2: host threads (bound to the device's NUMA node) that write the hits into the records
-	struct HostPool* pool = 0;
-	int trace_variant = 3;           // BVH2 traversal kernel: 0 generic, 3 octant switch, 4 persistent warps (see trace_bvh2.cu)
-	int small_mode = 0;              // warp-subtree kernel: bit 0 = fragments staged in shared memory, bit 1 = aggregated bin updates
+	HostSlot slot[TBVH_SLOTS];       // allocated by the first host batch call
 	int inst_idx_bits = 32;          // the host program's INST_IDX_BITS (tiny_bvh.h:118): 32 = TLAS hits store hit.inst, 4..31 = top bits of hit.prim
-	int hq_small = 16;               // BuildHQ: nodes of at most this many fragments go to the warp-per-subtree kernel (<= 256)
-	int hq_cluster = 16;             // BuildHQ: largest thread-block cluster a node of the level phase may get (1..16)
-	int small_t = 128;               // builder: subtrees of at most this many primitives go to the warp kernel (<= 256)
-	int build_ctas = 0;              // persistent large phase: CTAs per SM (0 = by scene size)
+	int small_t = 128;               // builder: subtrees of at most this many primitives go to the warp kernel (8..128; every value gives the same tree)
 	int build_mode = 0;              // BVH::Build large phase: 0 = one persistent cooperative launch (k_large_phase), 1 = one launch per stage and level
-	// ring of 8-byte device counters for kernels that pull work from a counter (one per launch, so launches on different
-	// streams never share one)
-	unsigned long long* d_counters = 0;
-	std::atomic<uint32_t> counter_next{ 0 };
 };
-#define TBVH_COUNTERS 256
 
 uint32_t tbvh_next_generation(); // process-wide: a value no handle has carried before (a recycled handle address cannot revalidate a stale TLAS)
 struct BlasLink { tbvh_bvh blas; uint32_t generation; }; // host side: what a TLAS was built over
@@ -143,7 +120,6 @@ __device__ __forceinline__ float key2f( uint32_t k ) { return __uint_as_float( (
 int bvh2_trace_launch( tbvh_bvh b, const void* d_rays, uint32_t stride, void* d_hits, uint32_t hit_stride, uint32_t* d_bits, uint64_t n, bool anyhit, cudaStream_t s, unsigned long long* d_stats );
 int cwbvh_trace_launch( tbvh_bvh b, const void* d_rays, uint32_t stride, void* d_hits, uint32_t hit_stride, uint32_t* d_bits, uint64_t n, bool anyhit, cudaStream_t s, unsigned long long* d_stats );
 int cw_make_trav( tbvh_bvh b, cudaStream_t s, int known_depth = -1 ); // known_depth < 0: measured on the device
-unsigned long long* ctx_next_counter( tbvh_ctx c ); // a zero-on-use 8-byte device counter from the context's ring (persistent-warp ray fetch)
 int build_sah_launch( tbvh_bvh b, float c_trav, float c_int, int flavour );
 int build_hq_launch( tbvh_bvh b, float c_trav, float c_int );
 int refit_launch( tbvh_bvh b, cudaStream_t s );

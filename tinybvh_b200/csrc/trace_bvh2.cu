@@ -27,13 +27,13 @@
 	tmina = fmaxf( fmaxf( tx1a, ty1a ), fmaxf( tz1a, 0.0f ) ), tminb = fmaxf( fmaxf( tx1b, ty1b ), fmaxf( tz1b, 0.0f ) ); \
 	tmaxa = fminf( fminf( tx2a, ty2a ), fminf( tz2a, tmax ) ), tmaxb = fminf( fminf( tx2b, ty2b ), fminf( tz2b, tmax ) );
 
-// MINB = minimum resident CTAs per SM asked of ptxas (10 -> 40 warps / SM without spills; 12 and 16 were measured slower).
+// 10 resident CTAs per SM asked of ptxas: 40 warps / SM without spills (12 and 16 were measured slower).
 // OCTSW = 1: when every ray of the warp lies in the same direction octant (the normal case for camera and shadow rays) the
 // slab tests run through an octant-specialised instance picked by a warp-uniform switch, which removes the 12 selects
 // per step; mixed warps use the generic per-lane selects.  Same arithmetic, same order, same results either way.
 // STACKN = traversal stack entries: TBVH_STACK (64) for trees of depth < 64, TBVH_STACK_DEEP (256, the reference's own stack, :3249) above.
-template <bool ANYHIT, bool STATS, int MINB, int OCTSW, int STACKN>
-__global__ void __launch_bounds__( 128, MINB ) k_trace_bvh2( const float4* __restrict__ nodes, const float4* __restrict__ tris,
+template <bool ANYHIT, bool STATS, int OCTSW, int STACKN>
+__global__ void __launch_bounds__( 128, 10 ) k_trace_bvh2( const float4* __restrict__ nodes, const float4* __restrict__ tris,
 	const char* rays, const uint32_t stride, char* hits, const uint32_t hit_stride, // may alias (in-place hits): plain loads
 	uint32_t* __restrict__ bits, const uint64_t n, const uint32_t root_ref, const uint32_t root_count,
 	unsigned long long* __restrict__ stats )
@@ -142,109 +142,6 @@ __global__ void __launch_bounds__( 128, MINB ) k_trace_bvh2( const float4* __res
 	}
 }
 
-// Persistent-warp variant for incoherent ray sets (diffuse bounces): resident warps pull rays from a global counter and
-// refill the lanes whose ray has terminated once at least REFILL_MIN lanes are idle, so a few long rays no longer hold 31
-// idle lanes hostage (the persistent-thread ray fetch of wavefront.cl:93-115, at lane granularity).  Each ray is still
-// traversed exactly as in k_trace_bvh2 - same order, same arithmetic - only the lane it runs on differs.
-#define PERSIST_ROUND 12     // traversal steps between two refill votes
-#define REFILL_MIN 6         // idle lanes needed before the warp pays for a refill
-template <bool ANYHIT>
-__global__ void __launch_bounds__( 128, 10 ) k_trace_bvh2_persist( const float4* __restrict__ nodes, const float4* __restrict__ tris,
-	const char* rays, const uint32_t stride, char* hits, const uint32_t hit_stride, uint32_t* bits, const uint64_t n,
-	const uint32_t root_ref, const uint32_t root_count, unsigned long long* next )
-{
-	const uint32_t lane = threadIdx.x & 31;
-	bool active = false, more = true;
-	uint64_t idx = 0;
-	float ox = 0, oy = 0, oz = 0, dx = 0, dy = 0, dz = 0, rdx = 0, rdy = 0, rdz = 0, nrox = 0, nroy = 0, nroz = 0;
-	float tmax = 0, hu = 0, hv = 0;
-	uint32_t hprim = 0, ref = 0, cnt = 0;
-	bool posX = true, posY = true, posZ = true;
-	uint2 stack[TBVH_STACK];
-	int sp = 0;
-	while (true)
-	{
-		const uint32_t idle = __ballot_sync( 0xffffffffu, !active );
-		if (more && (idle == 0xffffffffu || __popc( idle ) >= REFILL_MIN))
-		{
-			unsigned long long base = 0;
-			if (lane == 0) base = atomicAdd( next, (unsigned long long)__popc( idle ) );
-			base = __shfl_sync( 0xffffffffu, base, 0 );
-			if (base >= n) more = false; // warp-uniform: the pool is dry
-			if (!active)
-			{
-				idx = base + __popc( idle & ((1u << lane) - 1u) );
-				if (idx < n)
-				{
-					const float4* rp = (const float4*)(rays + idx * stride);
-					const float4 ro4 = rp[0], rd4 = rp[1], rr4 = rp[2], rh4 = rp[3];
-					ox = ro4.x, oy = ro4.y, oz = ro4.z, dx = rd4.x, dy = rd4.y, dz = rd4.z, rdx = rr4.x, rdy = rr4.y, rdz = rr4.z;
-					nrox = -__fmul_rn( ox, rdx ), nroy = -__fmul_rn( oy, rdy ), nroz = -__fmul_rn( oz, rdz );
-					posX = dx >= 0, posY = dy >= 0, posZ = dz >= 0;
-					tmax = rh4.x, hu = rh4.y, hv = rh4.z, hprim = __float_as_uint( rh4.w );
-					ref = root_ref, cnt = root_count, sp = 0, active = true;
-				}
-			}
-		}
-		if (!__any_sync( 0xffffffffu, active )) break;
-		if (active)
-		{
-			bool done = false, occluded = false;
-			for (int it = 0; it < PERSIST_ROUND && !done; it++)
-			{
-				bool pop = true;
-				if (cnt == 0)
-				{
-					const float4* p = nodes + (size_t)ref * 2;
-					const float4 a0 = __ldg( p ), a1 = __ldg( p + 1 ), b0 = __ldg( p + 2 ), b1 = __ldg( p + 3 );
-					float tmina, tminb, tmaxa, tmaxb;
-					{ SLAB_PAIR( posX, posY, posZ ) }
-					const bool hita = tmaxa >= tmina, hitb = tmaxb >= tminb;
-					const uint32_t refa = __float_as_uint( a0.w ), cnta = __float_as_uint( a1.w );
-					const uint32_t refb = __float_as_uint( b0.w ), cntb = __float_as_uint( b1.w );
-					if (hita && hitb)
-					{
-						const bool swp = tmina > tminb;
-						ref = swp ? refb : refa, cnt = swp ? cntb : cnta;
-						stack[sp++] = swp ? make_uint2( refa, cnta ) : make_uint2( refb, cntb );
-						pop = false;
-					}
-					else if (hita) ref = refa, cnt = cnta, pop = false;
-					else if (hitb) ref = refb, cnt = cntb, pop = false;
-				}
-				else
-				{
-					const float4* tp = tris + (size_t)ref * 3;
-					for (uint32_t k = 0; k < cnt; k++, tp += 3)
-					{
-						const float4 v0 = __ldg( tp ), e1 = __ldg( tp + 1 ), e2 = __ldg( tp + 2 );
-						float t, u, v;
-						if (mt_test( ox, oy, oz, dx, dy, dz, v0, e1, e2, tmax, t, u, v ))
-						{
-							if (ANYHIT) { occluded = true; break; }
-							tmax = t, hu = u, hv = v, hprim = __float_as_uint( v0.w );
-						}
-					}
-					if (ANYHIT && occluded) done = true;
-				}
-				if (pop && !done)
-				{
-					if (sp == 0) done = true;
-					else { const uint2 e = stack[--sp]; ref = e.x, cnt = e.y; }
-				}
-			}
-			if (done)
-			{
-				if (!ANYHIT) *(float4*)(hits + idx * hit_stride) = make_float4( tmax, hu, hv, __uint_as_float( hprim ) );
-				else if (occluded) atomicOr( bits + (idx >> 5), 1u << (uint32_t)(idx & 31) );
-				active = false;
-			}
-		}
-	}
-}
-
-unsigned long long* ctx_next_counter( tbvh_ctx c ) { return c->d_counters + (c->counter_next.fetch_add( 1 ) % TBVH_COUNTERS); }
-
 int bvh2_trace_launch( tbvh_bvh b, const void* d_rays, uint32_t stride, void* d_hits, uint32_t hit_stride, uint32_t* d_bits,
 	uint64_t n, bool anyhit, cudaStream_t s, unsigned long long* d_stats )
 {
@@ -256,32 +153,17 @@ int bvh2_trace_launch( tbvh_bvh b, const void* d_rays, uint32_t stride, void* d_
 	const uint32_t block = 128;
 	const uint64_t grid = (n + block - 1) / block;
 	if (grid > 0x7fffffffull) { tbvh_set_error( "ray batch too large for one launch" ); return TBVH_E_ARG; }
-	const int variant = b->ctx->trace_variant;
-	#define LAUNCH( A, S, M, O, D ) k_trace_bvh2<A, S, M, O, D><<<(uint32_t)grid, block, 0, s>>>( b->d_trav, b->d_leaf_tris, (const char*)d_rays, stride, \
+	// statistics launches run the per-lane slab step (OCTSW = 0), every other launch the octant switch
+	#define LAUNCH( A, S, O, D ) k_trace_bvh2<A, S, O, D><<<(uint32_t)grid, block, 0, s>>>( b->d_trav, b->d_leaf_tris, (const char*)d_rays, stride, \
 		(char*)d_hits, hit_stride, d_bits, n, root_ref, root_count, d_stats )
 	if (deep)
 	{
 		// depth 64..255: the same kernel with the reference's 256-entry stack (2 KiB of local memory per ray)
-		if (d_stats) { if (anyhit) LAUNCH( true, true, 10, 0, TBVH_STACK_DEEP ); else LAUNCH( false, true, 10, 0, TBVH_STACK_DEEP ); }
-		else { if (anyhit) LAUNCH( true, false, 10, 1, TBVH_STACK_DEEP ); else LAUNCH( false, false, 10, 1, TBVH_STACK_DEEP ); }
-		LAUNCHED();
-		return TBVH_OK;
+		if (d_stats) { if (anyhit) LAUNCH( true, true, 0, TBVH_STACK_DEEP ); else LAUNCH( false, true, 0, TBVH_STACK_DEEP ); }
+		else { if (anyhit) LAUNCH( true, false, 1, TBVH_STACK_DEEP ); else LAUNCH( false, false, 1, TBVH_STACK_DEEP ); }
 	}
-	if (variant == 4 && !d_stats)
-	{
-		// persistent warps: one resident wave (10 CTAs of 128 threads per SM), rays pulled from a counter that belongs to this launch
-		unsigned long long* next = ctx_next_counter( b->ctx );
-		CUDA_TRY( cudaMemsetAsync( next, 0, 8, s ) );
-		if (anyhit) CUDA_TRY( cudaMemsetAsync( d_bits, 0, ((n + 31) / 32) * 4, s ) );
-		const uint32_t pgrid = (uint32_t)b->ctx->sm_count * 10u;
-		if (anyhit) k_trace_bvh2_persist<true><<<pgrid, 128, 0, s>>>( b->d_trav, b->d_leaf_tris, (const char*)d_rays, stride, (char*)d_hits, hit_stride, d_bits, n, root_ref, root_count, next );
-		else k_trace_bvh2_persist<false><<<pgrid, 128, 0, s>>>( b->d_trav, b->d_leaf_tris, (const char*)d_rays, stride, (char*)d_hits, hit_stride, d_bits, n, root_ref, root_count, next );
-		LAUNCHED();
-		return TBVH_OK;
-	}
-	if (d_stats) { if (anyhit) LAUNCH( true, true, 10, 0, TBVH_STACK ); else LAUNCH( false, true, 10, 0, TBVH_STACK ); }
-	else if (variant == 3) { if (anyhit) LAUNCH( true, false, 10, 1, TBVH_STACK ); else LAUNCH( false, false, 10, 1, TBVH_STACK ); }
-	else { if (anyhit) LAUNCH( true, false, 10, 0, TBVH_STACK ); else LAUNCH( false, false, 10, 0, TBVH_STACK ); }
+	else if (d_stats) { if (anyhit) LAUNCH( true, true, 0, TBVH_STACK ); else LAUNCH( false, true, 0, TBVH_STACK ); }
+	else { if (anyhit) LAUNCH( true, false, 1, TBVH_STACK ); else LAUNCH( false, false, 1, TBVH_STACK ); }
 	#undef LAUNCH
 	LAUNCHED();
 	return TBVH_OK;

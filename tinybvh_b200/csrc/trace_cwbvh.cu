@@ -252,11 +252,11 @@ int cwbvh_trace_launch( tbvh_bvh b, const void* d_rays, uint32_t stride, void* d
 	const uint32_t block = 128;
 	const uint64_t grid = (n + block - 1) / block;
 	if (grid > 0x7fffffffull) { tbvh_set_error( "ray batch too large for one launch" ); return TBVH_E_ARG; }
-	const int sw = b->ctx->trace_variant == 0 ? 0 : 1; // trace_variant 0: the per-lane form only (A/B switch for measurements)
+	// statistics launches run the per-lane node step (OCTSW = 0), every other launch the octant switch
 	#define LAUNCH( A, S, O ) k_trace_wide<A, S, O><<<(uint32_t)grid, block, 0, s>>>( b->d_cw_trav, b->d_cw_tris, (const char*)d_rays, stride, \
 		(char*)d_hits, hit_stride, d_bits, n, d_stats )
-	if (anyhit) { if (d_stats) LAUNCH( true, true, 0 ); else if (sw) LAUNCH( true, false, 1 ); else LAUNCH( true, false, 0 ); }
-	else { if (d_stats) LAUNCH( false, true, 0 ); else if (sw) LAUNCH( false, false, 1 ); else LAUNCH( false, false, 0 ); }
+	if (anyhit) { if (d_stats) LAUNCH( true, true, 0 ); else LAUNCH( true, false, 1 ); }
+	else { if (d_stats) LAUNCH( false, true, 0 ); else LAUNCH( false, false, 1 ); }
 	#undef LAUNCH
 	LAUNCHED();
 	return TBVH_OK;

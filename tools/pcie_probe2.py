@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Developer probe: host-buffer path throughput (tbvh_intersect / tbvh_occluded on 128-byte host records) against where the ray
-buffer lives (NUMA-local or wherever the process happened to start) and the pipeline options.  A one-triangle scene makes the
+buffer lives (NUMA-local or wherever the process happened to start).  A one-triangle scene makes the
 traversal free, so the call time is transfer time.   python tools/pcie_probe2.py [n_rays_log2]"""
 import os
 import sys
@@ -66,33 +66,3 @@ h = api.pinned_empty(n, R.RAY_DTYPE, device=0)
 api.bind_to_device(0)
 fill(h)
 run("local pinned buffer", h)
-api.set_option("d2h_mode", 0)
-run("local, 16-byte rows back (d2h 0)", h)
-api.set_option("d2h_mode", 1)
-if "--short" in sys.argv:
-    sys.exit(0)
-api.set_option("host_path", 2)
-run("local, whole-record inbound", h)
-api.set_option("d2h_mode", 2)
-api.set_option("scatter_threads", 32)
-run("local, whole-record + scatter x32", h)
-api.set_option("d2h_mode", 0)
-api.set_option("host_path", 0)
-for thr in (32,):
-    api.set_option("d2h_mode", 2)
-    api.set_option("scatter_threads", thr)
-    run(f"local, host scatter x{thr}", h)
-api.set_option("d2h_mode", 0)
-if "--all" in sys.argv:
-    for key, val in (("chunk_rays", 1 << 18), ("chunk_rays", 1 << 20), ("chunk_rays", 1 << 19)):
-        api.set_option(key, val)
-        run(f"local, {key}={val}", h)
-    for sp in (2, 3):
-        api.set_option("h2d_split", sp)
-        run(f"local, h2d_split={sp}", h)
-    api.set_option("h2d_split", 1)
-    api.set_option("host_path", 1)
-    run("local, gather kernel inbound", h)
-    api.set_option("host_path", 0)
-    api.set_option("d2h_mode", 3)
-    run("local, scatter kernel outbound", h)

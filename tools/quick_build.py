@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Developer probe: GPU build time of a scene under the builder's tuning knobs (small_mode x small_t)."""
+"""Developer probe: GPU build time of a scene at the builder's switch points small_t (--all: 64 and 128)."""
 import os
 import sys
 
@@ -10,12 +10,10 @@ from tinybvh_b200 import api, scenes  # noqa: E402
 for scene in [a for a in sys.argv[1:] if not a.startswith("--")] or ["sponza"]:
     v, label = scenes.load_scene(scene)
     n = v.shape[0] // 3
-    for mode in ((0, 1, 2, 3) if "--all" in sys.argv else (0,)):
-        for t in ((64, 128) if "--all" in sys.argv else (128,)):
-            api.set_option("small_mode", mode)
-            api.set_option("small_t", t)
-            best = 1e9
-            for _ in range(3):
-                e = api.BVH().Build(v)
-                best = min(best, e.info().build_ms)
-            print(f"{label}: {n} tris small_mode {mode} small_t {t}: build {best:.3f} ms = {n / best / 1e3:.1f} Mtris/s  (nodes {e.info().used_nodes})", flush=True)
+    for t in ((64, 128) if "--all" in sys.argv else (128,)):
+        api.set_option("small_t", t)
+        best = 1e9
+        for _ in range(3):
+            e = api.BVH().Build(v)
+            best = min(best, e.info().build_ms)
+        print(f"{label}: {n} tris small_t {t}: build {best:.3f} ms = {n / best / 1e3:.1f} Mtris/s  (nodes {e.info().used_nodes})", flush=True)

@@ -35,8 +35,7 @@ def main():
     e = getattr(api.BVH(), builder)(v)
     e = getattr(api.BVH(), builder)(v)
     i = e.info()
-    print(f"{label}: {v.shape[0] // 3} tris, GPU build {i.build_ms:.3f} ms ({v.shape[0] // 3 / i.build_ms / 1e3:.1f} Mtris/s), nodes {i.used_nodes}, depth {i.max_depth}, "
-          f"variant {os.environ.get('TBVH_TRACE_VARIANT', '0')} small_t {os.environ.get('TBVH_SMALL_T', '256')}")
+    print(f"{label}: {v.shape[0] // 3} tris, GPU build {i.build_ms:.3f} ms ({v.shape[0] // 3 / i.build_ms / 1e3:.1f} Mtris/s), nodes {i.used_nodes}, depth {i.max_depth}")
     layout = sys.argv[3] if len(sys.argv) > 3 and not sys.argv[3].startswith("--") else "bvh"
     if layout == "cwbvh":
         import ctypes as C
@@ -60,12 +59,6 @@ def main():
     print(f"primary: {n} rays, {steps / n:.1f} steps/ray, {tris / n:.2f} tris/ray")
     best, med = timeit(lambda: e.Intersect(dprim, hits=hits))
     print(f"primary  closest: best {best:.3f} ms  {n / best / 1e3:.1f} Mrays/s (median {n / med / 1e3:.1f})")
-    if layout == "bvh":
-        for var in (0, 4):
-            api.set_option("trace_variant", var)
-            best, med = timeit(lambda: e.Intersect(dprim, hits=hits))
-            print(f"primary  closest variant {var}: best {best:.3f} ms  {n / best / 1e3:.1f} Mrays/s")
-        api.set_option("trace_variant", 3)
     # shadow + diffuse from traced primaries (host side generation)
     traced = prim.copy()
     h = hits.cpu().numpy()
@@ -84,14 +77,6 @@ def main():
     e.Intersect(ddf, hits=hits)
     steps, tris = e.get_stats()[:2]
     e.set_stats(False)
-    if layout == "bvh":
-        for var in (0, 4):
-            api.set_option("trace_variant", var)
-            best, med = timeit(lambda: e.IsOccluded(dsh, bits=bits))
-            print(f"shadow   anyhit  variant {var}: best {best:.3f} ms  {n / best / 1e3:.1f} Mrays/s")
-            best, med = timeit(lambda: e.Intersect(ddf, hits=hits))
-            print(f"diffuse  closest variant {var}: best {best:.3f} ms  {n / best / 1e3:.1f} Mrays/s")
-        api.set_option("trace_variant", 3)
     best, med = timeit(lambda: e.Intersect(ddf, hits=hits))
     print(f"diffuse  closest: best {best:.3f} ms  {n / best / 1e3:.1f} Mrays/s (median {n / med / 1e3:.1f})  {steps / n:.1f} steps/ray {tris / n:.2f} tris/ray")
     # host path (pinned) e2e
